@@ -264,7 +264,7 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
     const uint32_t stage_base = sbase + S::staging + quarter * (kStageBufs * kSlabBytes2);
     const bool issuer = kTrain && half == 0 && lane == 0;
     const uint32_t a_ready_leader = pair ? cluster_map_shared(bar_a_ready, 0) : bar_a_ready;
-    uint32_t acc_phase[2] = {0, 0};
+    uint32_t acc_phase = 0;  // bit r: parity of accumulator region r (a register, not a local array)
     uint32_t n_staged = 0;
     uint32_t titer = 0;
     for (int64_t tile; (tile = seq.get(titer)) >= 0; ++titer) {
@@ -281,8 +281,8 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
         const int epi = L.epi;
         const int nchunk = L.n_halves * 2;
         if (threadIdx.x == 0) FS_TRACE2(titer, g, 3);
-        mbar_wait(bar_acc_full + 8 * r, acc_phase[r]);
-        acc_phase[r] ^= 1;
+        mbar_wait(bar_acc_full + 8 * r, (acc_phase >> r) & 1u);
+        acc_phase ^= 1u << r;
         tc_fence_after();
         if (threadIdx.x == 0) FS_TRACE2(titer, g, 4);
         float part[3] = {0.f, 0.f, 0.f};
