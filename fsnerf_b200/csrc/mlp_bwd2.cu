@@ -10,7 +10,7 @@
 //                   PLACE as the next step's A operand; every finished chunk is handed to the
 //                   MMA warps and staged through smem per 32-row slab
 //      warps 8..11  store warps: copy each staged slab into the CTA's private ring of dpre
-//                   images (below)
+//                   images (below) and add its column sums to the layer's bias gradient
 //      warps 12,13  MMA issuers, alternating chunks (mlp_issue.cuh): D[128 x 256] = dpre . W
 //      warp 14      weight producers: two lanes, alternating W^T operand stages (L2 -> smem
 //                   bulk copies)
@@ -21,10 +21,8 @@
 //    dW[N_out x K_in] += dpre^T . X accumulated in TENSOR MEMORY over every tile it is dealt
 //    (jobs with several CTAs interleave the tiles) and flushed ONCE with fp32 atomics.  Both
 //    operands are [samples x features] SWIZZLE_128B images used MN-major: X from the forward
-//    stash (HBM, read once), dpre from the ring.  Eight more warps of the CTA take what the
-//    tensor core does not: the layer's bias gradient (column sums of the dpre slabs) and, in the
-//    two jobs that have the inputs in shared memory, the degenerate sigma / rgb head weight
-//    gradients (N = 1 / 3) on CUDA cores, all accumulated in registers over the whole launch.
+//    stash (HBM, read once), dpre from the ring.  Warps: 0 scout, 1 MMA issuer, 2..5 bulk-copy
+//    issuers that also flush the accumulator, 6 releaser; the others are idle.
 //
 //  The ring replaces round 1's full-size dstash workspace (4.9 KB/sample written by dgrad and
 //  read back by wgrad through HBM: 16 GB per C2 step).  Each dgrad CTA owns `depth` 64 KB
@@ -102,7 +100,6 @@ struct ArgsB {
 };
 // the dpre image ring shared by the two roles
 struct RingB {
-  int debug;        // FSNERF_DEBUG_FLAGS (tuning experiments only)
   uint32_t* tile_ctr;  // next unclaimed tile (dynamic scheduling of the dgrad CTAs)
   int32_t* tile_of;    // [n_d][row_cap]: tile claimed by dgrad CTA b for its iteration i, -1 past its last
   int row_cap;
@@ -115,14 +112,14 @@ struct RingB {
 };
 
 // ------------------------------------------------------------------ wgrad role layout
-constexpr int kSlabRows = 64;                     // samples per stage (32: measured 3.40 vs 3.34 ms; the side-warp paths assume 64)
+constexpr int kSlabRows = 64;                     // samples per stage (32: measured 3.40 vs 3.34 ms)
 constexpr int kSlabsPerTile = kTileM / kSlabRows;
 constexpr int kIssueLanes = 2 * kSlabsPerTile;    // issuing lanes of each of the four producer warps (8 threads per slab)
 constexpr int kSlabBytes = kSlabRows * 128;       // 8 KB per 64-feature chunk
 // A stage holds one 64-sample slab of the job's operands: (a_chunks + b_chunks) x 8 KB, so the
 // small jobs (encoding parts, branch) get a deeper ring out of the same 192 KB: their per-tile
 // work is a few hundred cycles and only tiles in flight hide the load latency.
-constexpr int kWRingBytes = 24 * 8192 + 3 * 2048;  // 3 stages of a [256 x 256] job (+ its out / d_out rows)
+constexpr int kWRingBytes = 24 * 8192;             // 3 stages of a [256 x 256] job
 constexpr int kWMaxStages = 8;
 constexpr int kWSmemBars = kWRingBytes;            // full[8], empty[8], acc_full, TMEM slot, queue counters
 constexpr int kWQueue = 64;                        // tile queue entries (scout -> issuers / releaser)
@@ -135,14 +132,10 @@ constexpr int kMaxJobs = kMaxGemm + 4;
 struct WgradJob {
   int a_img, a_chunks;  // dpre image index in the ring sequence, N_out / 64
   int b_off, b_chunks;  // input image (stash record), K_in(part) / 64
-  int c_off, c_chunks;  // one more stash image staged for the side warps only (rgb head input), 0: none
   int w_off, ld, col0, ncols, nrows;
   int cta_begin, n_split;
   int cons_inc;         // what this reader adds to cons[] per image (2 / readers of the image)
-  int bias_off;         // >= 0: this job also sums the dpre columns into grads[bias_off ...]
-  int head;             // 1: sigma head from the B slabs (last hidden layer's output); 2: rgb head from the C slabs
 };
-constexpr int kSideWarp0 = 7, kSideWarps = 8;  // wgrad role: warps 7..14
 struct WgradPlan {
   int n_jobs, n_ctas;
   WgradJob job[kMaxJobs];
@@ -154,11 +147,6 @@ constexpr int kSmemFused = SmemB::total > kWSmemTotal ? SmemB::total : kWSmemTot
 __device__ __forceinline__ uint32_t ld_acquire_u32(const uint32_t* p) {
   uint32_t v;
   asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ uint32_t ld_relaxed_u32(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
   return v;
 }
 __device__ __forceinline__ void st_release_u32(uint32_t* p, uint32_t v) {
@@ -227,7 +215,6 @@ __device__ __forceinline__ void dgrad_cta(uint8_t* smem, const MlpProgram& prog,
   volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(smem + BarsB::tmem_slot);
   const float* heads = reinterpret_cast<const float*>(smem + SmemB::heads);
   float* bias_acc = reinterpret_cast<float*>(smem + SmemB::bias);
-  const bool bias_here = (ring.debug & 8) == 0;  // FSNERF_DEBUG_FLAGS & 8: bias sums on the wgrad side warps instead (measured slower: 4.25 vs 3.42 ms)
   const int64_t n_tiles = (args.n_samples + kTileM - 1) / kTileM;
   // Tiles are claimed from a global counter (the ring manager keeps the feed two tiles ahead):
   // the dgrad CTAs do not run at the same speed (they are throttled by different wgrad CTAs and
@@ -286,9 +273,7 @@ __device__ __forceinline__ void dgrad_cta(uint8_t* smem, const MlpProgram& prog,
         while (n_claimed < want) {
           int t = -1;
           if (!dry && n_claimed < ring.row_cap - 1) {
-            // (FSNERF_DEBUG_FLAGS & 16: the static split blockIdx, blockIdx + n_d, ... for A/B runs)
-            const int64_t c = (ring.debug & 16) ? (int64_t)my_id + (int64_t)n_claimed * ring.n_d
-                                                : (int64_t)atomicAdd(ring.tile_ctr, 1u);
+            const int64_t c = atomicAdd(ring.tile_ctr, 1u);
             if (c < n_tiles) t = (int)c;
           }
           if (t < 0) dry = true;
@@ -322,8 +307,9 @@ __device__ __forceinline__ void dgrad_cta(uint8_t* smem, const MlpProgram& prog,
   } else if (warp >= kWarpRed0) {
     // ------------------------------------------------ store warps: ring images + bias gradients
     // one warp per lane quarter.  Per staged slab (32 rows x 64 features of one chunk): copy it
-    // into the current ring image and free the buffer (the bias gradients = column sums of these
-    // images are taken by the wgrad CTAs, which have every image in shared memory anyway).
+    // into the current ring image, add its column sums to the layer's bias gradient and free the
+    // buffer.  (Summing the columns on the wgrad CTAs, which have every image in shared memory
+    // anyway, was measured slower: 4.25 vs 3.42 ms.)
     const int quarter = warp - kWarpRed0;
     const uint32_t stage_base = sbase + SmemB::staging + quarter * (kStageBufsB * kSlabBytesB);
     uint8_t* my_ring = ring.base + (size_t)my_id * ring.depth * kImgSlotBytes;
@@ -367,7 +353,7 @@ __device__ __forceinline__ void dgrad_cta(uint8_t* smem, const MlpProgram& prog,
 #pragma unroll
             for (int k = 0; k < 8; ++k) dst[k * 32 + lane] = t[k];
           }
-          if (bias_here) {
+          {
             float s0 = 0.f, s1 = 0.f, c0 = 0.f, c1 = 0.f;
             const uint8_t* a = smem + SmemB::staging + quarter * (kStageBufsB * kSlabBytesB) + b * kSlabBytesB + ((lane & 3) << 2);
             const uint32_t unit = (uint32_t)lane >> 2;
@@ -539,12 +525,11 @@ __device__ __forceinline__ void dgrad_cta(uint8_t* smem, const MlpProgram& prog,
   __syncthreads();
   if (stats && threadIdx.x == 0) stats[0] = clock64() - t_begin;
   if (warp == kWarpMmaB) tmem_dealloc(tmem_base, 512);
-  if (bias_here)  // bias gradients of this CTA -> global
-    for (int g = 0; g < prog.n_gemm; ++g) {
-      const int ncols = prog.layer[g].n_halves * 128;
-      if ((int)threadIdx.x < ncols)
-        atomicAdd(args.grads + prog.layer[g].bias_off + threadIdx.x, bias_acc[g * 256 + threadIdx.x]);
-    }
+  for (int g = 0; g < prog.n_gemm; ++g) {  // bias gradients of this CTA -> global
+    const int ncols = prog.layer[g].n_halves * 128;
+    if ((int)threadIdx.x < ncols)
+      atomicAdd(args.grads + prog.layer[g].bias_off + threadIdx.x, bias_acc[g * 256 + threadIdx.x]);
+  }
 }
 
 // =========================================================================== wgrad role
@@ -567,7 +552,6 @@ __device__ __forceinline__ void wgrad_cta(uint8_t* smem, const MlpProgram& prog,
   while (j + 1 < plan.n_jobs && cta >= plan.job[j + 1].cta_begin) ++j;
   const WgradJob& J = plan.job[j];
   const int part = cta - J.cta_begin;
-  const int64_t n_tiles = (args.n_samples + kTileM - 1) / kTileM;
   // This CTA reads the images of dgrad CTAs part, part + n_split, ... (every tile of theirs), in
   // whatever order they are published: a consumer bound to a fixed tile order would stall on one
   // late producer while the others fill their rings and stall too.
@@ -587,18 +571,14 @@ __device__ __forceinline__ void wgrad_cta(uint8_t* smem, const MlpProgram& prog,
   };
   long long* stats = args.trace ? args.trace + kStatBase + 8 * (ring.n_d + cta) : nullptr;
   const long long t_begin = stats ? clock64() : 0;
-  // head jobs also stage the slab's rows of out / d_out (fp32 [P,4]): 1 KB each behind the operand chunks
-  const uint32_t aux_off = (uint32_t)(J.a_chunks + J.b_chunks + J.c_chunks) * kSlabBytes;
-  const uint32_t stage_bytes = aux_off + (J.head ? 2048u : 0u);
-  const bool side = J.bias_off >= 0 || J.head != 0;
-  // tile of the slab held by each stage (written by issuing thread 0 before it arms the barrier)
-  volatile uint32_t* stage_tile = reinterpret_cast<volatile uint32_t*>(smem + kWSmemBars + 176);
+  const int n_cp = J.a_chunks + J.b_chunks;  // operand chunks per stage
+  const uint32_t stage_bytes = (uint32_t)n_cp * kSlabBytes;
   volatile long long* issue_clk = reinterpret_cast<volatile long long*>(smem + kWSmemQueue + kWQueue * 8);  // stats only
   const uint32_t n_stages = (kWRingBytes / stage_bytes) < (uint32_t)kWMaxStages ? (kWRingBytes / stage_bytes) : (uint32_t)kWMaxStages;
   if (threadIdx.x == 0) {
     for (int s = 0; s < kWMaxStages; ++s) {
       mbar_init(bar_full + 8 * s, 8);   // the eight issuing threads of a slab (four lanes of two producer warps)
-      mbar_init(bar_empty + 8 * s, side ? 2 + kSideWarps : 2);  // MMA commit + releaser (+ side warps)
+      mbar_init(bar_empty + 8 * s, 2);  // MMA commit + releaser
     }
     mbar_init(bar_acc_full, 1);
     *ready_upto = 0;
@@ -625,7 +605,6 @@ __device__ __forceinline__ void wgrad_cta(uint8_t* smem, const MlpProgram& prog,
       // its stage's barrier for its own bytes: at most one or two copies per thread and tile.
       const int pw = (warp - 2) * kIssueLanes + lane;  // issuing thread index (lanes 0..kIssueLanes-1 issue)
       const int my_slab = ((warp - 2) * kIssueLanes) >> 3, my_c = pw & 7;  // (one slab per warp or per warp pair)
-      const int n_cp = J.a_chunks + J.b_chunks + J.c_chunks;
       uint32_t fenced_upto = 0;
       StatClock pc{0, stats != nullptr && warp == 2 && lane == 0};
       long long st_ready = 0, st_empty = 0;
@@ -652,24 +631,12 @@ __device__ __forceinline__ void wgrad_cta(uint8_t* smem, const MlpProgram& prog,
           const uint32_t q = (bi >> 8) * (uint32_t)ring.n_img + (uint32_t)J.a_img;
           const uint8_t* a_img = ring.base + ((size_t)b * ring.depth + q % (uint32_t)ring.depth) * kImgSlotBytes;
           const uint8_t* b_img = args.stash + (size_t)tile * prog.stash_tile_bytes + J.b_off;
-          const uint8_t* c_img = args.stash + (size_t)tile * prog.stash_tile_bytes + J.c_off;
           if (b == 0 && pw == 0 && J.cons_inc == 2) evt(args.trace, EVT_ISSUE, q);
           const uint32_t sa = sbase + stage * stage_bytes, sb = sa + (uint32_t)J.a_chunks * kSlabBytes;
           int mine = 0;
           for (int c = my_c; c < n_cp; c += 8) ++mine;
-          if (my_c == 0) {
-            stage_tile[stage] = (uint32_t)tile;  // ordered before the arrive below (release)
-            if (stats) issue_clk[stage] = clock64();
-          }
-          uint32_t aux_bytes = 0;
-          const int64_t p0 = tile * kTileM + my_slab * kSlabRows;
-          if (J.head && my_c == 7 && p0 < args.n_samples)
-            aux_bytes = (uint32_t)((args.n_samples - p0 < kSlabRows) ? (args.n_samples - p0) : kSlabRows) * 16u;
-          mbar_arrive_expect_tx(bar_full + 8 * stage, (uint32_t)mine * kSlabBytes + (J.head == 2 ? 2u : 1u) * aux_bytes);
-          if (aux_bytes) {
-            bulk_g2s(sa + aux_off + 1024, args.d_out + 4 * p0, aux_bytes, bar_full + 8 * stage);
-            if (J.head == 2) bulk_g2s(sa + aux_off, args.out + 4 * p0, aux_bytes, bar_full + 8 * stage);
-          }
+          if (my_c == 0 && stats) issue_clk[stage] = clock64();
+          mbar_arrive_expect_tx(bar_full + 8 * stage, (uint32_t)mine * kSlabBytes);
           // (L2 eviction hints — evict_first on the stash stream, evict_last on the ring reads and
           // writes — recover the 10-slot ring's loss against the 5-slot one, 4.00 -> 3.75 ms, and
           // add nothing to the 5-slot ring: it is resident without them)
@@ -677,115 +644,14 @@ __device__ __forceinline__ void wgrad_cta(uint8_t* smem, const MlpProgram& prog,
             if (c < J.a_chunks)
               bulk_g2s(sa + c * kSlabBytes, a_img + c * kChunkBytes + my_slab * kSlabBytes, kSlabBytes,
                        bar_full + 8 * stage);
-            else if (c < J.a_chunks + J.b_chunks)
+            else
               bulk_g2s(sb + (c - J.a_chunks) * kSlabBytes, b_img + (c - J.a_chunks) * kChunkBytes + my_slab * kSlabBytes,
                        kSlabBytes, bar_full + 8 * stage);
-            else
-              bulk_g2s(sb + (c - J.a_chunks) * kSlabBytes,
-                       c_img + (c - J.a_chunks - J.b_chunks) * kChunkBytes + my_slab * kSlabBytes, kSlabBytes,
-                       bar_full + 8 * stage);
           }
         }
         __syncwarp();
       }
       if (pc.on) { stats[1] = st_ready; stats[2] = st_empty; }
-    } else if (warp >= kSideWarp0 && warp < kSideWarp0 + kSideWarps && side) {
-      // ------------------------------------------------ side warps (CUDA cores)
-      // Every slab of the job is in shared memory for at least the duration of its MMAs.  Warp sw
-      // takes chunk (sw & 3) and rows 32 * (sw >> 2) .. +32 of the 64-row slab; lane l owns the
-      // feature pair (2l, 2l+1) of that chunk (conflict-free 4 B reads of the SW128 rows).
-      const int sw = warp - kSideWarp0;
-      const int ch = sw & 3, r0 = (sw >> 2) * 32;
-      const uint32_t lane_off = (uint32_t)(lane & 3) << 2;
-      const uint32_t unit = (uint32_t)lane >> 2;
-      float b0 = 0.f, b1 = 0.f;                        // bias gradient (column sums of dpre)
-      float s0 = 0.f, s1 = 0.f, sb_sum = 0.f;          // sigma head
-      float rg[3][2] = {{0.f, 0.f}, {0.f, 0.f}, {0.f, 0.f}}, rb[3] = {0.f, 0.f, 0.f};  // rgb head
-      // rgb head: the C image is 128 wide (2 chunks): warp sw takes chunk (sw & 1), rows 16 * (sw >> 1) .. +16
-      const int ch2 = sw & 1, r2 = (sw >> 1) * 16;
-      uint32_t cnt = 0;
-      StatClock xc{0, stats != nullptr && sw == 0 && lane == 0};
-      long long st_busy = 0;
-      for (uint32_t n = 0; have_tile(n); ++n) {
-        for (int slab = 0; slab < kTileM / kSlabRows; ++slab, ++cnt) {
-          const uint32_t stage = cnt % n_stages, phase = (cnt / n_stages) & 1;
-          mbar_wait(bar_full + 8 * stage, phase);
-          xc.start();
-          const int64_t p0 = (int64_t)stage_tile[stage] * kTileM + slab * kSlabRows;
-          // plain loads (the barrier wait above is the compiler fence): a volatile asm per load
-          // would serialise the loop on the 29-cycle shared-memory latency
-          const uint8_t* st = smem + stage * stage_bytes;
-          const int64_t n_valid = args.n_samples - p0;  // rows of this slab that are real samples
-          if (J.bias_off >= 0 && ch < J.a_chunks) {
-            const uint8_t* a = st + ch * kSlabBytes + lane_off + r0 * 128;
-            float c0 = 0.f, c1 = 0.f;
-#pragma unroll
-            for (int i = 0; i < 32; i += 2) {
-              const uint32_t w0 = *reinterpret_cast<const uint32_t*>(a + i * 128 + ((unit ^ (uint32_t)(i & 7)) << 4));
-              const uint32_t w1 = *reinterpret_cast<const uint32_t*>(a + (i + 1) * 128 + ((unit ^ (uint32_t)((i + 1) & 7)) << 4));
-              b0 += bf16_lo(w0); b1 += bf16_hi(w0);
-              c0 += bf16_lo(w1); c1 += bf16_hi(w1);
-            }
-            b0 += c0; b1 += c1;
-          }
-          if (J.head == 1) {  // d(sigma weight)[k] += dsigma[s] * h[s][k]
-            const uint8_t* hrow = st + (J.a_chunks + ch) * kSlabBytes + lane_off + r0 * 128;
-            const uint8_t* drow = st + aux_off + 1024 + r0 * 16 + 12;
-            float c0 = 0.f, c1 = 0.f, cs = 0.f;
-#pragma unroll
-            for (int i = 0; i < 32; i += 2) {
-              const float d0 = (r0 + i < n_valid) ? *reinterpret_cast<const float*>(drow + i * 16) : 0.f;
-              const float d1 = (r0 + i + 1 < n_valid) ? *reinterpret_cast<const float*>(drow + (i + 1) * 16) : 0.f;
-              const uint32_t w0 = *reinterpret_cast<const uint32_t*>(hrow + i * 128 + ((unit ^ (uint32_t)(i & 7)) << 4));
-              const uint32_t w1 = *reinterpret_cast<const uint32_t*>(hrow + (i + 1) * 128 + ((unit ^ (uint32_t)((i + 1) & 7)) << 4));
-              s0 = fmaf(d0, bf16_lo(w0), s0); s1 = fmaf(d0, bf16_hi(w0), s1);
-              c0 = fmaf(d1, bf16_lo(w1), c0); c1 = fmaf(d1, bf16_hi(w1), c1);
-              cs += d0 + d1;
-            }
-            s0 += c0; s1 += c1;
-            if (ch == 0) sb_sum += cs;  // every lane of the two chunk-0 warps holds the same sum
-          } else if (J.head == 2) {  // d(rgb weight)[c][k] += dz[s][c] * hb[s][k]
-            const uint8_t* xrow = st + (J.a_chunks + J.b_chunks + ch2) * kSlabBytes + lane_off + r2 * 128;
-            const uint8_t* orow = st + aux_off + r2 * 16;
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-              const float4 o4 = *reinterpret_cast<const float4*>(orow + i * 16);
-              const float4 g4 = *reinterpret_cast<const float4*>(orow + 1024 + i * 16);
-              const bool ok = r2 + i < n_valid;
-              const float dz0 = ok ? g4.x * o4.x * (1.0f - o4.x) : 0.f;
-              const float dz1 = ok ? g4.y * o4.y * (1.0f - o4.y) : 0.f;
-              const float dz2 = ok ? g4.z * o4.z * (1.0f - o4.z) : 0.f;
-              const uint32_t w = *reinterpret_cast<const uint32_t*>(xrow + i * 128 + ((unit ^ (uint32_t)((r2 + i) & 7)) << 4));
-              const float x0 = bf16_lo(w), x1 = bf16_hi(w);
-              rg[0][0] = fmaf(dz0, x0, rg[0][0]); rg[0][1] = fmaf(dz0, x1, rg[0][1]);
-              rg[1][0] = fmaf(dz1, x0, rg[1][0]); rg[1][1] = fmaf(dz1, x1, rg[1][1]);
-              rg[2][0] = fmaf(dz2, x0, rg[2][0]); rg[2][1] = fmaf(dz2, x1, rg[2][1]);
-              if (ch2 == 0) { rb[0] += dz0; rb[1] += dz1; rb[2] += dz2; }
-            }
-          }
-          __syncwarp();
-          if (lane == 0) mbar_arrive(bar_empty + 8 * stage);
-          xc.stop(st_busy);
-        }
-      }
-      if (xc.on) stats[7] = st_busy;
-      // one atomic per feature and warp at the very end
-      if (J.bias_off >= 0 && ch < J.a_chunks) {
-        atomicAdd(args.grads + J.bias_off + 64 * ch + 2 * lane, b0);
-        atomicAdd(args.grads + J.bias_off + 64 * ch + 2 * lane + 1, b1);
-      }
-      if (J.head == 1) {
-        atomicAdd(args.grads + prog.sigma_w_off + 64 * ch + 2 * lane, s0);
-        atomicAdd(args.grads + prog.sigma_w_off + 64 * ch + 2 * lane + 1, s1);
-        if (ch == 0 && lane == 0) atomicAdd(args.grads + prog.sigma_b_off, sb_sum);
-      } else if (J.head == 2) {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-          atomicAdd(args.grads + prog.rgb_w_off + c * 128 + 64 * ch2 + 2 * lane, rg[c][0]);
-          atomicAdd(args.grads + prog.rgb_w_off + c * 128 + 64 * ch2 + 2 * lane + 1, rg[c][1]);
-          if (ch2 == 0 && lane == 0) atomicAdd(args.grads + prog.rgb_b_off + c, rb[c]);
-        }
-      }
     } else if (warp == 6) {
       // releaser: once the last slab of a tile has landed, the whole dpre image is in shared
       // memory and its ring slot goes back to the dgrad CTA.  It also arrives on the stage's
@@ -1113,13 +979,6 @@ int job_overhead_cycles() {
   if (v < 0) v = env_int("FSNERF_BWD_JOB_OVERHEAD", 3000);
   return v;
 }
-// Measured: the two heads are ~4800 CUDA-core cycles per tile (issue bound), which the branch /
-// connection jobs cannot absorb without several more CTAs; their own small kernel is faster.
-bool fuse_heads() {
-  static int v = -1;
-  if (v < 0) v = env_int("FSNERF_BWD_FUSE_HEADS", 0);
-  return v != 0;
-}
 // tile_of rows: a dgrad CTA may claim up to 4x its even share (then it stops claiming)
 int tile_row_cap(int64_t n_tiles, int n_d) { return (int)(4 * ((n_tiles + n_d - 1) / n_d) + 8); }
 int64_t tile_table_bytes(int64_t n_tiles, int n_d) {
@@ -1222,16 +1081,16 @@ extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* param
   ha.n_samples = n_samples; ha.n_tiles = n_tiles; ha.out = out; ha.d_out = d_out;
   ha.g_sigma_w = grads + P.sigma_w_off; ha.g_sigma_b = grads + P.sigma_b_off;
   ha.g_rgb_w = grads + P.rgb_w_off; ha.g_rgb_b = grads + P.rgb_b_off;
-  // one resident wave (3 CTAs per SM): 0.203 vs 0.218 ms per C2 step with two waves, 0.237 with three
+  // one resident wave (3 CTAs per SM): 0.203 vs 0.218 ms per C2 step with two waves, 0.237 with three.
+  // (On the wgrad CTAs' idle warps the heads cost ~4800 CUDA-core cycles per tile, more than the
+  // jobs that stage their inputs can absorb: measured 6.4-9.4 ms per launch against 0.22 ms here.)
   const int hgrid = (int)(n_tiles < 3 * kNumSMs ? n_tiles : 3 * kNumSMs);
-  if (!fuse_heads()) {
-    {
-      FsProfScope prof_("mlp_heads_wgrad", stream);
-      mlp_heads_wgrad_kernel<<<hgrid, 256, 0, st>>>(ha);
-    }
-    rc = fsnerf_check_launch("mlp_backward(heads)");
-    if (rc != FSNERF_OK) return rc;
+  {
+    FsProfScope prof_("mlp_heads_wgrad", stream);
+    mlp_heads_wgrad_kernel<<<hgrid, 256, 0, st>>>(ha);
   }
+  rc = fsnerf_check_launch("mlp_backward(heads)");
+  if (rc != FSNERF_OK) return rc;
 
   // ---- dgrad plan + issue table
   PlanB PL;
@@ -1279,7 +1138,7 @@ extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* param
   for (int s = 0; s < PL.n_steps; ++s)
     if ((s & 1) == ((PL.n_steps - 1) & 1)) ++T.last_acc_n;
 
-  // ---- wgrad plan: (layer, input part) jobs, CTAs split proportionally to the bytes they stream
+  // ---- wgrad plan: (layer, input part) jobs, CTAs split in proportion to their cycles per tile
   WgradPlan WP;
   WP.n_jobs = 0;
   double cost[kMaxJobs], total = 0;
@@ -1296,15 +1155,6 @@ extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* param
       J.a_img = P.n_gemm - 1 - g; J.a_chunks = a_chunks;
       J.w_off = L.w_off; J.ld = L.ld; J.nrows = L.n_halves * 128;
       J.cons_inc = 2 / readers[g];
-      J.c_off = 0; J.c_chunks = 0; J.head = 0;
-      // the layer's bias gradient rides on its lighter job; the heads on the jobs that stage their inputs
-      J.bias_off = ((part == 1 || !L.use_aux) && (env_int("FSNERF_DEBUG_FLAGS", 0) & 8)) ? L.bias_off : -1;
-      if (fuse_heads()) {  // FSNERF_BWD_FUSE_HEADS=1: the heads on the side warps instead of their own kernel
-        if (L.epi == EPI_CONN && part == 0) J.head = 1;  // B = the last hidden layer's output
-        if (L.epi == EPI_BRANCH && part == 1) {          // C = the branch layer's own output image
-          J.head = 2; J.c_off = L.stash_off; J.c_chunks = L.n_halves * 2;
-        }
-      }
       if (part == 0) {
         J.b_off = P.layer[g - 1].stash_off; J.b_chunks = L.n_act_chunks;
         J.col0 = 0; J.ncols = L.n_act_chunks * 64;
@@ -1314,7 +1164,7 @@ extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* param
       }
       // cycles a wgrad CTA spends per tile: its MMAs (M = 128 per a-chunk pair, N = 64 per
       // b-chunk: N/2 cycles per K = 16 step, 8 steps per tile) plus a per-tile overhead that the
-      // stage ring does not hide (measured ~600 cycles)
+      // stage ring does not hide (swept 0-12000 cycles: 1500 is ~15 % slower, 3000 and up are flat)
       cost[WP.n_jobs] = (J.a_chunks / 2) * 8 * (J.b_chunks * 32) + job_overhead_cycles();
       total += cost[WP.n_jobs];
       ++WP.n_jobs;
@@ -1361,7 +1211,6 @@ extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* param
   RG.n_d = sp.n_d;
   RG.depth = ring_depth_for(P.n_gemm);
   RG.n_img = P.n_gemm;
-  RG.debug = env_int("FSNERF_DEBUG_FLAGS", 0);
   uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
   RG.prod = reinterpret_cast<uint32_t*>(ws);
   RG.tile_ctr = RG.prod + 255;

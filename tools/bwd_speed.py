@@ -1,4 +1,4 @@
-"""Per-kernel times of one training step (tuning aid; honours FSNERF_DEBUG_FLAGS)."""
+"""Per-kernel times of one training step (tuning aid)."""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from fsnerf_b200 import ops
@@ -44,4 +44,4 @@ for _ in range(n):
 prof = ops.profile_read()
 ops.profile_enable(False)
 print({k: v[1] // n for k, v in prof.items() if k.startswith("mlp")}, end=" ")
-print(f"FSNERF_DEBUG_FLAGS={os.environ.get('FSNERF_DEBUG_FLAGS','0')}:", {k: round(v[0] / n, 3) for k, v in sorted(prof.items(), key=lambda kv: -kv[1][0])[:5]})
+print({k: round(v[0] / n, 3) for k, v in sorted(prof.items(), key=lambda kv: -kv[1][0])[:5]})

@@ -47,7 +47,7 @@ for j in sorted(set(int(x) for x in (wg[:, 6] * 1e3).round().tolist())):
     m = (wg[:, 6] * 1e3).round() == j
     r = wg[m]
     print(f"  job {j:2d}: {int(m.sum()):3d} {r[:, 4].mean() * 1e3:7.0f} {r[:, 0].mean():9.1f} {r[:, 1].mean():9.1f} "
-          f"{r[:, 2].mean():9.1f} {r[:, 3].mean():9.1f} {(r[:, 5] / (2 * r[:, 4])).mean():9.0f} side-busy {r[:, 7].mean():9.1f}")
+          f"{r[:, 2].mean():9.1f} {r[:, 3].mean():9.1f} {(r[:, 5] / (2 * r[:, 4])).mean():9.0f}")
 
 # life of the first images of dgrad CTA 0 (global timer, us relative to the first event)
 e = trace.cpu()[4096:4096 + 7 * 256].view(7, 256).double()

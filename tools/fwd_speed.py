@@ -1,4 +1,4 @@
-"""MLP forward throughput (render-style, no stash) — tuning aid; honours FSNERF_DEBUG_FLAGS."""
+"""MLP forward throughput (render-style, no stash) — tuning aid."""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from fsnerf_b200 import ops
@@ -22,4 +22,4 @@ for _ in range(n):
 e1.record(); torch.cuda.synchronize()
 ms = e0.elapsed_time(e1) / n
 tf = R * S * 1186816 / (ms * 1e-3) / 1e12
-print(f"FSNERF_DEBUG_FLAGS={os.environ.get('FSNERF_DEBUG_FLAGS','0')}: {ms:.3f} ms, {tf:.0f} TFLOP/s, {tf/1408.5:.3f} of sustained peak")
+print(f"{ms:.3f} ms, {tf:.0f} TFLOP/s, {tf/1408.5:.3f} of sustained peak")

@@ -29,11 +29,3 @@ for it in range(1, 3):
     for s in range(9):
         r = [int(x) - t0 if x > 0 else -1 for x in t[it, s, :6]]
         print(f"  tile {it} step {s}: mma wait {r[1]-r[0]:6d} issue {r[2]-r[1]:6d} | epi wait(acc) {r[4]-r[3]:6d} epi {r[5]-r[4]:6d} | abs {r}")
-
-d = trace.cpu()[512:512 + 16 * 8].view(4, 4, 8)
-print("epilogue warp 0 detail, tile 1: [ld issue+mask ldg | slab wait | ld wait | alu | sttm+arrive | stage out]")
-for s_ in range(4):
-    for c in range(4):
-        r = [int(x) for x in d[s_, c]]
-        if r[0] > 0:
-            print(f"  step {s_} chunk {c}: {r[1]-r[0]:5d} {r[2]-r[1]:5d} {r[3]-r[2]:5d} {r[4]-r[3]:5d} {r[5]-r[4]:5d} {r[6]-r[5]:5d} | start {r[0]-t0}")

@@ -34,21 +34,11 @@ _lib.load().fsnerf_debug_set_trace(_lib.ptr(trace))
 run()
 torch.cuda.synchronize()
 _lib.load().fsnerf_debug_set_trace(None)
-tall = trace.cpu()
-t = tall[:512].view(4, 16, 8)
+t = trace.cpu()[:512].view(4, 16, 8)
 t0 = int(t[t > 0].min())
 print("columns: mma_wait_start mma_start mma_committed | epi_wait_start epi_start epi_end   (cycles since first event; fine pass overwrites coarse)")
 for it in range(3):
-    print(f"tile iter {it}: encode start {int(t[it,15,6])-t0} end {int(t[it,15,7])-t0}")
+    print(f"tile iter {it}:")
     for g_ in range(10):
         r = [int(x) - t0 if x > 0 else -1 for x in t[it, g_, :6]]
         print(f"  L{g_}: mma wait {r[1]-r[0]:6d} issue {r[2]-r[1]:6d} | epi wait(acc) {r[4]-r[3]:6d} epi {r[5]-r[4]:6d} | abs {r}")
-
-d = tall[512:512 + 10 * 5 * 8].view(10, 5, 8)
-if int(d.max()) > 0:
-    print("MMA warp detail, tile iter 1: per chunk  [top->waits done | ->MMA0 issued | ->MMA1,probes,MMA2 | ->MMA3 | ] ok_a/ok_w at top; abs top")
-    for g_ in range(10):
-        for c in range(5):
-            r = [int(x) for x in d[g_, c]]
-            if r[0] > 0 and r[4] > 0:
-                print(f"  L{g_} chunk{c}: waits {r[1]-r[0]:5d} mma0 {r[2]-r[1]:5d} mma1+probes+mma2 {r[3]-r[2]:5d} mma3 {r[4]-r[3]:5d} | ok {r[7]} | top {r[0]-t0}")
