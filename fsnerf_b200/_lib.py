@@ -43,6 +43,8 @@ SIGNATURES = {
                                           _i, _f, _f, _f, _p, _p]),
     "fsnerf_encode": (_i, [_l, _i, _i, _p, _p, _p, _p, _p]),
     "fsnerf_occgrid_march": (_i, [_l, _p, _p, _p, _f, _f, _f, _p, _i, _i, _p, _p, _p, _p, _p, _p, _p]),
+    "fsnerf_occgrid_filter": (_i, [_l, _p, _p, _p, _p, _f, _f, _p, _p, _p, _p, _p, _p]),
+    "fsnerf_packed_points": (_i, [_l, _p, _p, _p, _p, _p, _p, _p, _p]),
     "fsnerf_composite_packed_forward": (_i, [_l, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
     "fsnerf_composite_packed_backward": (_i, [_l, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
     "fsnerf_occgrid_update": (_i, [_l, _p, _p, _f, _p, _p, _p]),

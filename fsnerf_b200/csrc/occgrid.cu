@@ -131,6 +131,20 @@ __global__ void __launch_bounds__(kWarps * 32) occgrid_march_kernel(const MarchA
 }
 
 // ------------------------------------------------------------------ packed compositing
+// One 32-sample block of a ray: the lane's optical depth sd = sigma * delta, alpha = 1 - exp(-sd)
+// and transmittance T = exp(-(optical depth of every earlier sample of the ray)).  carry holds the
+// ray's optical depth before the block and advances past it.  Lanes past the end pass sigma = 0 and
+// t0 = t1 = 0.  The compositing forward and the visibility filter both call this, so the filter
+// thresholds exactly the T / alpha the compositor reports.
+__device__ __forceinline__ void packed_block_trans(float sigma, float t0, float t1, int lane, float& carry,
+                                                   float& alpha, float& T) {
+  const float sd = sigma * (t1 - t0);
+  alpha = 1.0f - expf(-sd);
+  const float incl = warp_incl_scan_add(sd, lane);
+  T = expf(-(carry + (incl - sd)));
+  carry += __shfl_sync(0xffffffffu, incl, 31);
+}
+
 __global__ void __launch_bounds__(kWarps * 32)
 composite_packed_fwd_kernel(int64_t n_rays, const int64_t* __restrict__ offsets, const float4* __restrict__ raw,
                             const float* __restrict__ ts, const float* __restrict__ te,
@@ -152,11 +166,8 @@ composite_packed_fwd_kernel(int64_t n_rays, const int64_t* __restrict__ offsets,
       t0 = __ldg(ts + base + s);
       t1 = __ldg(te + base + s);
     }
-    const float sd = c.w * (t1 - t0);
-    const float alpha = 1.0f - expf(-sd);
-    const float incl = warp_incl_scan_add(sd, lane);
-    const float T = expf(-(carry + (incl - sd)));
-    carry += __shfl_sync(0xffffffffu, incl, 31);
+    float alpha, T;
+    packed_block_trans(c.w, t0, t1, lane, carry, alpha, T);
     const float w = T * alpha;
     if (s < S) {
       weights[base + s] = w;
@@ -178,6 +189,67 @@ composite_packed_fwd_kernel(int64_t n_rays, const int64_t* __restrict__ offsets,
     rgb[r * 3] = acc_r; rgb[r * 3 + 1] = acc_g; rgb[r * 3 + 2] = acc_b;
     opacity[r] = acc_w;
     depth[r] = acc_d;
+  }
+}
+
+// Visibility filter of OccGridEstimator.sampling (nerfacc's transmittance test): sample i of a ray
+// is kept iff T_i >= early_stop_eps and, when alpha_thre > 0, alpha_i >= alpha_thre.  sigma is the
+// raw density head and may be negative, so T can rise again along a ray: the kept set is not a
+// prefix, and each block is compacted by ballot.  Count pass (out_offsets NULL) writes counts[r];
+// the fill pass writes the survivors in their original order from out_offsets[r] on.
+__global__ void __launch_bounds__(kWarps * 32)
+occgrid_filter_kernel(int64_t n_rays, const int64_t* __restrict__ offsets, const float* __restrict__ ts,
+                      const float* __restrict__ te, const float* __restrict__ sigmas, float early_stop_eps,
+                      float alpha_thre, const int64_t* __restrict__ out_offsets, int32_t* __restrict__ counts,
+                      int64_t* __restrict__ ray_indices, float* __restrict__ ts_out, float* __restrict__ te_out) {
+  const int lane = threadIdx.x & 31;
+  const int64_t r = (int64_t)blockIdx.x * kWarps + (threadIdx.x >> 5);
+  if (r >= n_rays) return;
+  const int64_t base = offsets[r];
+  const int S = (int)(offsets[r + 1] - base);
+  const int64_t out_base = out_offsets ? out_offsets[r] : 0;
+  float carry = 0.f;
+  int total = 0;
+  for (int s0 = 0; s0 < S; s0 += 32) {
+    const int s = s0 + lane;
+    float sigma = 0.f, t0 = 0.f, t1 = 0.f;
+    if (s < S) {
+      sigma = __ldg(sigmas + base + s);
+      t0 = __ldg(ts + base + s);
+      t1 = __ldg(te + base + s);
+    }
+    float alpha, T;
+    packed_block_trans(sigma, t0, t1, lane, carry, alpha, T);
+    const bool keep = s < S && T >= early_stop_eps && (alpha_thre <= 0.f || alpha >= alpha_thre);
+    const unsigned m = __ballot_sync(0xffffffffu, keep);
+    if (out_offsets && keep) {
+      const int64_t p = out_base + total + __popc(m & ((1u << lane) - 1u));
+      ray_indices[p] = r;
+      ts_out[p] = t0;
+      te_out[p] = t1;
+    }
+    total += __popc(m);
+  }
+  if (!out_offsets && lane == 0) counts[r] = total;
+}
+
+// x[i] = o[r] + ((d[r] * (t_starts[i] + t_ends[i])) / 2), r = ray_indices[i]: the operation order of
+// the drop-in's torch expression (src/render/rendering.py:58-84), rounded op by op with no FMA
+// contraction, so x is bit-identical to it.  (torch divides by a scalar through its reciprocal;
+// * 0.5 and / 2 round identically.)
+__global__ void packed_points_kernel(int64_t n, const int64_t* __restrict__ ray_indices,
+                                     const float* __restrict__ ts, const float* __restrict__ te,
+                                     const float* __restrict__ rays_o, const float* __restrict__ rays_d,
+                                     float* __restrict__ x, float* __restrict__ dirs) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int64_t r = ray_indices[i];
+  const float sum = __fadd_rn(__ldg(ts + i), __ldg(te + i));
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    const float d = __ldg(rays_d + 3 * r + k);
+    x[3 * i + k] = __fadd_rn(__ldg(rays_o + 3 * r + k), __fmul_rn(__fmul_rn(d, sum), 0.5f));
+    if (dirs) dirs[3 * i + k] = d;
   }
 }
 
@@ -287,6 +359,32 @@ extern "C" int fsnerf_occgrid_march(int64_t n_rays, const float* rays_o, const f
   FsProfScope prof_("occgrid_march", stream);
   occgrid_march_kernel<<<(unsigned)((n_rays + kWarps - 1) / kWarps), kWarps * 32, 0, (cudaStream_t)stream>>>(a);
   return fsnerf_check_launch("occgrid_march");
+}
+
+extern "C" int fsnerf_occgrid_filter(int64_t n_rays, const int64_t* offsets, const float* t_starts,
+                                     const float* t_ends, const float* sigmas, float early_stop_eps,
+                                     float alpha_thre, const int64_t* out_offsets, int32_t* counts,
+                                     int64_t* ray_indices, float* out_t_starts, float* out_t_ends, void* stream) {
+  if (n_rays == 0) return FSNERF_OK;
+  FS_REQUIRE(n_rays > 0 && offsets, "occgrid_filter: bad n_rays / null offsets");
+  FS_REQUIRE((out_offsets && ray_indices && out_t_starts && out_t_ends) || (!out_offsets && counts),
+             "occgrid_filter: count pass needs counts; fill pass needs out_offsets and the three outputs");
+  FsProfScope prof_("occgrid_filter", stream);
+  occgrid_filter_kernel<<<(unsigned)((n_rays + kWarps - 1) / kWarps), kWarps * 32, 0, (cudaStream_t)stream>>>(
+      n_rays, offsets, t_starts, t_ends, sigmas, early_stop_eps, alpha_thre, out_offsets, counts, ray_indices,
+      out_t_starts, out_t_ends);
+  return fsnerf_check_launch("occgrid_filter");
+}
+
+extern "C" int fsnerf_packed_points(int64_t n, const int64_t* ray_indices, const float* t_starts,
+                                    const float* t_ends, const float* rays_o, const float* rays_d, float* x,
+                                    float* dirs, void* stream) {
+  if (n == 0) return FSNERF_OK;
+  FS_REQUIRE(n > 0 && ray_indices && t_starts && t_ends && rays_o && rays_d && x, "packed_points: null pointer");
+  FsProfScope prof_("packed_points", stream);
+  packed_points_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n, ray_indices, t_starts,
+                                                                                       t_ends, rays_o, rays_d, x, dirs);
+  return fsnerf_check_launch("packed_points");
 }
 
 extern "C" int fsnerf_composite_packed_forward(int64_t n_rays, const int64_t* offsets, const float* raw,

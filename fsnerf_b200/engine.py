@@ -8,6 +8,10 @@ Train step (src/run-nerf.py:232-285 with the sampler replaced per north_star):
   gen_rays* -> stratified -> coarse MLP -> composite -> sample_pdf -> fine MLP
   -> composite -> MSE grads -> composite bwd x2 -> MLP bwd x2 (heads + one fused
   dgrad/wgrad launch each) -> [NCCL all-reduce of the flat gradient] -> Adam on the flat buffer.
+With sampler="occgrid" (the reference's own sampler, src/run-nerf.py:92-98,288-295):
+  occgrid_march -> packed_points -> density MLP -> occgrid_filter -> packed_points -> MLP
+  -> packed composite -> MSE grads -> packed composite bwd -> MLP bwd -> [all-reduce] -> Adam
+  -> grid update every 16th step.
 Coarse and fine networks live in ONE flat fp32 parameter/gradient/moment buffer
 so the data-parallel exchange is a single collective (SURVEY.md §8e).
 """
@@ -20,6 +24,7 @@ from . import ops
 from ._lib import FsnerfError
 from .core.models import NeRF, freq_mask
 from .parallel import allreduce_gradients, loss_grad_scale
+from .render.rendering import OccGridEstimator
 
 _M64 = (1 << 64) - 1
 
@@ -36,21 +41,39 @@ def jitter_seeds(seed: int, rank: int, draw: int):
     return keys
 
 
+def grid_seed(seed: int, step: int) -> int:
+    """Key of the occupancy-grid update of train step `step`: (seed, step) only, never the rank,
+    so every rank of a data-parallel run draws the same cells and points and holds the same grid."""
+    return jitter_seeds(seed, 0, -1 - step)[0]
+
+
 class HotPath:
+    """sampler="hierarchical" (default): stratified + sample_pdf, coarse and fine networks.
+    sampler="occgrid": the reference's own configuration (src/run-nerf.py:92-98,232-295): ONE
+    network, an owned render.rendering.OccGridEstimator(roi_aabb, grid_resolution, grid_levels) for the
+    grid, fixed-step marching (render_step_size, near 0, far 1e10) with the transmittance visibility
+    filter (early_stop_eps 1e-4, alpha_thre 0) on a density-only forward, then a training forward of
+    the survivors.  Its train_step reads two sizes on the host: N (candidates) and M (survivors).
+    near / far / n_coarse / n_fine do not apply to it."""
+
     def __init__(self, n_coarse=64, n_fine=128, near=2.0, far=6.0, white_bkgd=True, device="cuda",
                  n_layers=8, d_hidden=256, skip=(4,), n_freqs=10, n_freqs_dir=4, log_space=True,
-                 seed=42, lr=5e-4, process_group=None, world_size=None):
+                 seed=42, lr=5e-4, process_group=None, world_size=None, sampler="hierarchical",
+                 roi_aabb=None, grid_resolution=128, grid_levels=1, render_step_size=5e-3):
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise FsnerfError("HotPath: CUDA device required (no CPU path)")
+        if sampler not in ("hierarchical", "occgrid"):
+            raise FsnerfError(f"HotPath: unknown sampler {sampler!r} (hierarchical | occgrid)")
         ops.require_device(self.device.index if self.device.index is not None else torch.cuda.current_device())
+        self.occgrid = sampler == "occgrid"
         self.n_coarse, self.n_fine = int(n_coarse), int(n_fine)
         self.near, self.far, self.white_bkgd = float(near), float(far), bool(white_bkgd)
         self.cfg = ops.make_cfg(n_layers, d_hidden, skip, n_freqs, n_freqs_dir, log_space)
         self.layout = ops.mlp_param_layout(self.cfg)
         self.names = ops.state_dict_names(self.cfg)
         self.n_net = ops.mlp_param_count(self.cfg)
-        self.hier = self.n_fine > 0
+        self.hier = self.n_fine > 0 and not self.occgrid
         n_nets = 2 if self.hier else 1
         kw = {"pos_fn": {"n_freqs": n_freqs, "log_space": log_space},
               "dir_fn": {"n_freqs": n_freqs_dir, "log_space": log_space}}
@@ -62,9 +85,13 @@ class HotPath:
             for i in range(n_nets):
                 net = NeRF(3, 3, n_layers, d_hidden, list(skip), **kw)
                 self.params[i * self.n_net:(i + 1) * self.n_net].copy_(net.flat_parameters())
-        # gradient buffer with the two loss accumulators behind it: ONE fill zeroes both every step
-        self._grads_and_loss = torch.zeros(self.params.numel() + 2, device=self.device)
+        # gradient buffer with the two loss accumulators behind it: ONE fill zeroes both every step.
+        # The occgrid sampler puts this rank's trained survivor count between them, so the gradient
+        # all-reduce also tells every rank whether any rank trained (one collective, one decision).
+        n_grad = self.params.numel() + (1 if self.occgrid else 0)
+        self._grads_and_loss = torch.zeros(n_grad + 2, device=self.device)
         self.grads = self._grads_and_loss[:self.params.numel()]
+        self._reduced = self._grads_and_loss[:n_grad]
         self.m = torch.zeros_like(self.params)
         self.v = torch.zeros_like(self.params)
         self.packed = [torch.empty(ops.mlp_packed_bytes(self.cfg), dtype=torch.uint8, device=self.device)
@@ -81,7 +108,7 @@ class HotPath:
                 torch.distributed.is_available() and torch.distributed.is_initialized()) else 1
         self.rank = torch.distributed.get_rank(process_group) if self.world > 1 and (
             torch.distributed.is_available() and torch.distributed.is_initialized()) else 0
-        self.loss_sums = self._grads_and_loss[self.params.numel():]
+        self.loss_sums = self._grads_and_loss[n_grad:]
         # in-step regularisers (SURVEY.md §8 f2): occlusion (src/core/loss.py:26-60) fused into the
         # compositing backward, weight-norm penalty (src/run-nerf.py:266-279) fused into Adam
         self.occ_sum = torch.zeros(1, device=self.device)
@@ -91,6 +118,16 @@ class HotPath:
         self._buf = {}
         self._packed_fresh = False
         self.launches = 0  # kernels of ours launched (bench.py reports it)
+        if self.occgrid:
+            if roi_aabb is None:
+                raise FsnerfError("HotPath(sampler='occgrid') needs roi_aabb")
+            self.estimator = OccGridEstimator(roi_aabb, resolution=int(grid_resolution),
+                                              levels=int(grid_levels)).to(self.device)
+            self.render_step_size = float(render_step_size)
+            self.early_stop_eps, self.alpha_thre = 1e-4, 0.0  # OccGridEstimator.sampling's defaults
+            self.k = 0  # train_step calls so far: the reference's loop counter (src/run-nerf.py:288-295)
+            self._grid_gen = torch.Generator(device=self.device)
+            self.last_counts = (0, 0)  # (candidates N, survivors M) of the last occgrid forward
 
     # ------------------------------------------------------------------ helpers
     def net_params(self, i):
@@ -177,10 +214,70 @@ class HotPath:
         out.update(ts_f=ts_f, te_f=te_f, raw_f=raw_f, rgb=rgb_f, opacity=op_f, depth=dp_f, w_f=w_f, st_f=st_f)
         return out
 
+    def _forward_occgrid(self, rays_o, rays_d, u, train):
+        """occgrid sampler: march -> density forward of the candidates -> visibility filter -> forward
+        of the survivors (stashed when train) -> packed compositing.  u: per-ray jitter U[0,1) or None.
+        Every step matches render.rendering.render_rays on OccGridEstimator bit for bit (same kernels,
+        same operands), including its answer to exactly one survivor (src/render/rendering.py:97-103):
+        a constant background, zero opacity and depth, and no raw samples to train."""
+        cfg, R = self.cfg, rays_o.shape[0]
+        self._pack()
+        est, step = self.estimator, self.render_step_size
+        near_planes = None if u is None else u * step  # the drop-in's 0 + u * step, bit for bit
+        ri, ts, te, offsets = ops.occgrid_march(rays_o, rays_d, est.binaries.view(torch.uint8), est.aabbs, step,
+                                                near=0.0, far=1e10, near_planes=near_planes)
+        N = ts.numel()
+        self.launches += 2
+        if N > 0:
+            x, _ = ops.packed_points(ri, ts, te, rays_o, rays_d)
+            sigmas = ops.mlp_forward(cfg, self.net_params(0), self.packed[0], x=x, mask_pos=self.mask_pos,
+                                     mask_dir=self.mask_dir, density_only=1)
+            ri, ts, te, offsets = ops.occgrid_filter(ts, te, offsets, sigmas, self.early_stop_eps, self.alpha_thre)
+            self.launches += 4
+        M = ts.numel()
+        self.last_counts = (N, M)
+        out = dict(ri=ri, ts=ts, te=te, offsets=offsets, M=M, raw=None, st=None)
+        if M == 1:
+            bk = 1.0 if self.white_bkgd else 0.0
+            out.update(rgb=torch.full((R, 3), bk, device=self.device), opacity=torch.zeros(R, 1, device=self.device),
+                       depth=torch.zeros(R, 1, device=self.device))
+            return out
+        if M > 0:
+            x, dirs = ops.packed_points(ri, ts, te, rays_o, rays_d, want_dirs=True)
+            out["st"] = self._bytes("stash", ops.mlp_stash_bytes(cfg, M)) if train else None
+            raw = ops.mlp_forward(cfg, self.net_params(0), self.packed[0], x=x, dirs=dirs, mask_pos=self.mask_pos,
+                                  mask_dir=self.mask_dir, stash=out["st"])
+            self.launches += 2
+        else:
+            raw = torch.zeros(0, 4, device=self.device)
+        rgb, op, dp, _, tr, _ = ops.composite_packed_forward(raw, ts, te, offsets, bkgd=self.bkgd)
+        self.launches += 1
+        out.update(raw=raw, trans=tr, rgb=rgb, opacity=op, depth=dp)
+        return out
+
+    def _occ_eval(self, x):
+        """occ_eval_fn of the reference's grid update: density of the current weights x step size"""
+        self._pack()
+        sigma = ops.mlp_forward(self.cfg, self.net_params(0), self.packed[0], x=x, mask_pos=self.mask_pos,
+                                mask_dir=self.mask_dir, density_only=1)
+        return sigma * self.render_step_size
+
+    @torch.no_grad()
+    def update_grid(self, step: int) -> None:
+        """occgrid sampler: OccGridEstimator.update_every_n_steps(step) (src/run-nerf.py:288-295; updates
+        when step % 16 == 0) with occ_eval_fn = density of the current weights x render_step_size.  The
+        cells and points are drawn from grid_seed(seed, step), so equal weights give equal grids."""
+        self._grid_gen.manual_seed(grid_seed(self._seed, step))
+        self.estimator.update_every_n_steps(step=step, occ_eval_fn=self._occ_eval, occ_thre=1e-2,
+                                            generator=self._grid_gen)
+
     @torch.no_grad()
     def render(self, rays_o, rays_d):
         """deterministic (eval) render of a ray chunk -> rgb[R,3], opacity[R,1], depth[R,1]"""
-        o = self._forward(rays_o, rays_d, None, None, train=False)
+        if self.occgrid:
+            o = self._forward_occgrid(rays_o, rays_d, None, train=False)
+        else:
+            o = self._forward(rays_o, rays_d, None, None, train=False)
         return o["rgb"], o["opacity"], o["depth"]
 
     # --------------------------------------------------------------- train step
@@ -201,6 +298,9 @@ class HotPath:
         penalty of src/run-nerf.py:266-279 ('l1' or Frobenius) on every network of the flat
         buffer; the caller applies the reference's `k < int(reg_ratio*Td)` gate by passing
         None.  self.reg_sums holds sum|w| (l1) / sum w^2 (l2) per regularised tensor."""
+        if self.occgrid:
+            return self._train_step_occgrid(rays_o, rays_d, rgb_gt, u_strat, lr, global_rays, apply_update,
+                                            occ_reg, weight_reg)
         cfg, R = self.cfg, rays_o.shape[0]
         G = int(global_rays) if global_rays is not None else R * self.world
         o = self._forward(rays_o, rays_d, u_strat, u_pdf, train=True, seeds=self._jitter_seeds())
@@ -241,6 +341,60 @@ class HotPath:
                 ops.adam_step(self.params, self.grads, self.m, self.v, self.lr if lr is None else lr, self.step)
                 self.launches += 1
             self._packed_fresh = False
+        return self.loss_sums
+
+    def _train_step_occgrid(self, rays_o, rays_d, rgb_gt, u, lr, global_rays, apply_update, occ_reg, weight_reg):
+        """train_step of the occgrid sampler: the step of examples/train_dropin.py --sampler occgrid
+        (src/run-nerf.py:232-295) on the fused kernels.  u: explicit per-ray jitter [R] (else drawn
+        in-kernel from the step's stratified key).  The loss goes to loss_sums[0].  The host reads
+        two sizes, N and M (ops.occgrid_march / ops.occgrid_filter); a data-parallel rank that
+        trained nothing also reads the all-reduced survivor count.
+
+        Fewer than two survivors (the empty grid of the first steps, or the one-survivor
+        background fallback) write no MLP gradient; when that holds on every rank, Adam does not
+        step and its step count stays, as torch.optim.Adam skips parameters whose .grad is None.
+        With apply_update the grid update of loop step k (the number of earlier train_step calls)
+        follows on the fresh weights."""
+        if occ_reg is not None:
+            raise FsnerfError("HotPath(sampler='occgrid'): occ_reg is not fused into the packed backward")
+        cfg, R = self.cfg, rays_o.shape[0]
+        G = int(global_rays) if global_rays is not None else R * self.world
+        k, self.k = self.k, self.k + 1
+        seed = self._jitter_seeds()[0]
+        if u is None:
+            u = ops.rng_uniform(R, seed, device=self.device)
+            self.launches += 1
+        o = self._forward_occgrid(rays_o, rays_d, u, train=True)
+        self._grads_and_loss.zero_()
+        M = o["M"]
+        trained = M >= 2
+        d_rgb = ops.mse_loss_grad(o["rgb"], rgb_gt, loss_grad_scale(G), self.loss_sums[0:1], want_grad=trained)
+        self.launches += 1
+        if trained:
+            d_raw, _ = ops.composite_packed_backward(o["raw"], o["ts"], o["te"], o["offsets"], o["trans"], d_rgb,
+                                                     bkgd=self.bkgd)
+            ws = self._bytes("bwd_ws", ops.mlp_bwd_workspace_bytes(cfg, M))
+            ops.mlp_backward(cfg, self.net_params(0), self.packed[0], M, o["st"], o["raw"], d_raw, self.net_grads(0),
+                             ws)
+            self._reduced[-1:].fill_(float(M))
+            self.launches += 3
+        any_trained = trained
+        if self.world > 1:
+            allreduce_gradients(self._reduced, self.pg)
+            if not trained:
+                any_trained = float(self._reduced[-1].item()) > 0
+        if apply_update:
+            if any_trained:
+                self.step += 1
+                if weight_reg is not None:
+                    ops.adam_step_reg(self.params, self.grads, self.m, self.v, self.lr if lr is None else lr,
+                                      self.step, weight_reg[0], weight_reg[1], self.reg_segs, self.reg_sums)
+                    self.launches += 2
+                else:
+                    ops.adam_step(self.params, self.grads, self.m, self.v, self.lr if lr is None else lr, self.step)
+                    self.launches += 1
+                self._packed_fresh = False
+            self.update_grid(k)
         return self.loss_sums
 
     @staticmethod

@@ -211,6 +211,51 @@ def occgrid_march(rays_o, rays_d, binaries, aabbs, step, near=0.0, far=1e10, nea
     return ri, ts, te, offsets
 
 
+def occgrid_filter(t_starts, t_ends, offsets, sigmas, early_stop_eps=1e-4, alpha_thre=0.0):
+    """Transmittance visibility filter of OccGridEstimator.sampling on packed candidates (ray r owns
+    [offsets[r], offsets[r+1])).  -> survivors' (ray_indices int64 [M], t_starts [M], t_ends [M],
+    offsets int64 [R+1]); two launches (count, fill) around one exclusive scan, one host read of M."""
+    ts, te, sig = _f32c(t_starts, "t_starts"), _f32c(t_ends, "t_ends"), _f32c(sigmas, "sigmas").reshape(-1)
+    if offsets.dtype != torch.int64 or offsets.dim() != 1 or offsets.numel() < 1:
+        raise _lib.FsnerfError("occgrid_filter: offsets must be int64 [R+1]")
+    R, N, dev = offsets.numel() - 1, ts.numel(), ts.device
+    if te.numel() != N or sig.numel() != N:
+        raise _lib.FsnerfError(f"occgrid_filter: t_starts / t_ends / sigmas sizes {N} / {te.numel()} / {sig.numel()}")
+    offsets = offsets.contiguous()
+    out_offsets = torch.zeros(R + 1, dtype=torch.int64, device=dev)
+    if N == 0 or R == 0:
+        return torch.empty(0, dtype=torch.int64, device=dev), ts.new_empty(0), ts.new_empty(0), out_offsets
+    counts = torch.empty(R, dtype=torch.int32, device=dev)
+    lib = _lib.load()
+    args = (R, ptr(offsets), ptr(ts), ptr(te), ptr(sig), float(early_stop_eps), float(alpha_thre))
+    check(lib.fsnerf_occgrid_filter(*args, None, ptr(counts), None, None, None, _stream()), "fsnerf_occgrid_filter")
+    torch.cumsum(counts, 0, out=out_offsets[1:])
+    M = int(out_offsets[-1].item())  # survivor count: the filter's one host read
+    ri = torch.empty(M, dtype=torch.int64, device=dev)
+    ts_o, te_o = torch.empty(M, device=dev), torch.empty(M, device=dev)
+    if M > 0:
+        check(lib.fsnerf_occgrid_filter(*args, ptr(out_offsets), None, ptr(ri), ptr(ts_o), ptr(te_o), _stream()),
+              "fsnerf_occgrid_filter")
+    return ri, ts_o, te_o, out_offsets
+
+
+def packed_points(ray_indices, t_starts, t_ends, rays_o, rays_d, want_dirs=False):
+    """-> x [N,3] = rays_o[ri] + rays_d[ri] * (t_starts + t_ends)[:, None] / 2 (bit-identical to that torch
+    expression) and, with want_dirs, dirs [N,3] = rays_d[ri] (else None)."""
+    ts, te = _f32c(t_starts, "t_starts"), _f32c(t_ends, "t_ends")
+    rays_o, rays_d = _f32c(rays_o, "rays_o"), _f32c(rays_d, "rays_d")
+    N, dev = ts.numel(), ts.device
+    if ray_indices.dtype != torch.int64 or ray_indices.numel() != N or te.numel() != N:
+        raise _lib.FsnerfError("packed_points: ray_indices must be int64 with one entry per interval")
+    if rays_o.shape != rays_d.shape or rays_o.dim() != 2 or rays_o.shape[1] != 3:
+        raise _lib.FsnerfError(f"packed_points: rays must be [R,3], got {tuple(rays_o.shape)} / {tuple(rays_d.shape)}")
+    x = torch.empty(N, 3, device=dev)
+    dirs = torch.empty(N, 3, device=dev) if want_dirs else None
+    check(_lib.load().fsnerf_packed_points(N, ptr(ray_indices.contiguous()), ptr(ts), ptr(te), ptr(rays_o),
+                                           ptr(rays_d), ptr(x), ptr(dirs), _stream()), "fsnerf_packed_points")
+    return x, dirs
+
+
 def offsets_from_ray_indices(ray_indices, n_rays):
     """[R+1] int64 segment offsets of sorted packed ray indices"""
     counts = torch.bincount(ray_indices, minlength=n_rays)

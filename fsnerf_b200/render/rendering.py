@@ -313,47 +313,44 @@ class OccGridEstimator(nn.Module):
         ri, ts, te, offsets = ops.occgrid_march(rays_o, rays_d, self.binaries.view(torch.uint8), self.aabbs,
                                                 render_step_size, far=far_plane, near_planes=near_planes)
         if (alpha_thre > 0.0 or early_stop_eps > 0.0) and sigma_fn is not None:
-            alpha_thre = min(alpha_thre, self.occs.mean().item())
+            if alpha_thre > 0.0:  # min(alpha_thre, mean) <= 0 disables the alpha test either way
+                alpha_thre = min(alpha_thre, self.occs.mean().item())
             sigmas = sigma_fn(ts, te, ri) if ts.numel() else ts.new_empty(0)
             assert sigmas.shape == ts.shape, f"sigmas must have shape of (N,)! Got {tuple(sigmas.shape)}"
-            raw = torch.zeros(ts.numel(), 4, device=dev)
-            raw[:, 3] = sigmas
-            *_, trans, alphas = ops.composite_packed_forward(raw, ts, te, offsets)
-            masks = trans >= early_stop_eps
-            if alpha_thre > 0.0:
-                masks = masks & (alphas >= alpha_thre)
-            ri, ts, te = ri[masks], ts[masks], te[masks]
+            ri, ts, te, _ = ops.occgrid_filter(ts, te, offsets, sigmas, early_stop_eps, alpha_thre)
         return ri, ts, te
 
     @torch.no_grad()
     def update_every_n_steps(self, step: int, occ_eval_fn=None, occ_thre: float = 1e-2, ema_decay: float = 0.95,
-                             warmup_steps: int = 256, n: int = 16) -> None:
+                             warmup_steps: int = 256, n: int = 16, generator: Optional[torch.Generator] = None) -> None:
+        """generator: draws the cell subset and the in-cell points (torch's default generator when None)"""
         if not self.training:
             raise RuntimeError("You should only call this function only during training. Please call "
                                "_update() directly if you want to update the field during inference.")
         if step % n == 0 and self.training:
-            self._update(step, occ_eval_fn, occ_thre, ema_decay, warmup_steps)
+            self._update(step, occ_eval_fn, occ_thre, ema_decay, warmup_steps, generator=generator)
 
-    def _sample_cells(self, step, warmup_steps, lvl):
+    def _sample_cells(self, step, warmup_steps, lvl, generator=None):
         """cell ids evaluated this round: all during warm-up, else 1/4 uniform + up to 1/4 occupied"""
         dev = self.occs.device
         if step < warmup_steps:
             return None
         n = self.cells_per_lvl // 4
-        uniform = torch.randint(self.cells_per_lvl, (n,), device=dev)
+        uniform = torch.randint(self.cells_per_lvl, (n,), device=dev, generator=generator)
         occupied = torch.nonzero(self.binaries[lvl].flatten())[:, 0]
         if occupied.numel() > n:
-            occupied = occupied[torch.randint(occupied.numel(), (n,), device=dev)]
+            occupied = occupied[torch.randint(occupied.numel(), (n,), device=dev, generator=generator)]
         return torch.cat([uniform, occupied])
 
     @torch.no_grad()
-    def _update(self, step, occ_eval_fn, occ_thre=1e-2, ema_decay=0.95, warmup_steps=256, rand=None) -> None:
+    def _update(self, step, occ_eval_fn, occ_thre=1e-2, ema_decay=0.95, warmup_steps=256, rand=None,
+                generator=None) -> None:
         res, dev = self.resolution, self.occs.device
         for lvl in range(self.levels):
-            ids = self._sample_cells(step, warmup_steps, lvl)
+            ids = self._sample_cells(step, warmup_steps, lvl, generator)
             flat = torch.arange(self.cells_per_lvl, device=dev) if ids is None else ids
             coords = torch.stack([flat // (res * res), (flat // res) % res, flat % res], -1).float()
-            u = torch.rand(coords.shape, device=dev) if rand is None else rand[lvl]
+            u = torch.rand(coords.shape, device=dev, generator=generator) if rand is None else rand[lvl]
             x = (coords + u) / res
             x = self.aabbs[lvl, :3] + x * (self.aabbs[lvl, 3:] - self.aabbs[lvl, :3])
             occ = occ_eval_fn(x).reshape(-1)

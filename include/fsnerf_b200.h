@@ -139,6 +139,23 @@ int fsnerf_occgrid_march(int64_t n_rays, const float* rays_o, const float* rays_
                          const float* aabbs, int levels, int res, const uint8_t* binaries,
                          const int64_t* offsets, int32_t* counts, int64_t* ray_indices,
                          float* t_starts, float* t_ends, void* stream);
+/* Visibility filter of OccGridEstimator.sampling (src/render/rendering.py:58-84 passes the
+ * density-only sigma_fn; nerfacc's filter keeps a sample iff its transmittance T >= early_stop_eps
+ * and, when alpha_thre > 0, alpha >= alpha_thre).  Candidates: ray r owns [offsets[r], offsets[r+1])
+ * of t_starts / t_ends / sigmas [N]; T and alpha are bit-identical to
+ * fsnerf_composite_packed_forward's trans / alphas of the same sigmas.  sigma may be negative, so
+ * the survivors are compacted per ray, not cut at a prefix.  Count pass: out_offsets == NULL,
+ * writes counts[n_rays].  Fill pass: out_offsets = exclusive scan of counts; writes the survivors'
+ * ray_indices (int64), t_starts, t_ends in their original order. */
+int fsnerf_occgrid_filter(int64_t n_rays, const int64_t* offsets, const float* t_starts,
+                          const float* t_ends, const float* sigmas, float early_stop_eps, float alpha_thre,
+                          const int64_t* out_offsets, int32_t* counts, int64_t* ray_indices,
+                          float* out_t_starts, float* out_t_ends, void* stream);
+/* Sample points of packed intervals (src/render/rendering.py:58-84):
+ * x[i] = rays_o[r] + rays_d[r] * (t_starts[i] + t_ends[i]) / 2 with r = ray_indices[i], rounded in
+ * that operation order without FMA contraction; dirs[i] = rays_d[r] when dirs is not NULL. */
+int fsnerf_packed_points(int64_t n, const int64_t* ray_indices, const float* t_starts, const float* t_ends,
+                         const float* rays_o, const float* rays_d, float* x, float* dirs, void* stream);
 /* nerfacc.volrend.rendering (src/render/rendering.py:89-96) on packed samples: ray r owns
  * [offsets[r], offsets[r+1]); raw [N,4] = (rgb, sigma).  Outputs rgb [R,3], opacity [R],
  * depth [R], weights [N]; trans / alphas [N] optional (trans is what the backward reads). */
