@@ -143,55 +143,6 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src, uin
       "l"(src), "r"(bytes), "r"(bar)
       : "memory");
 }
-// ---------------------------------------------------------------- thread-block clusters (CTA pairs)
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-// all threads of every CTA of the cluster (also a CTA-wide barrier)
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// address of `smem_addr` (a shared::cta address of this CTA) in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t cluster_map_shared(uint32_t smem_addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(rank));
-  return r;
-}
-// arrive on a barrier of any CTA of the cluster (address from cluster_map_shared)
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// Same without the release: a cluster-scope release is a full memory fence (measured: the
-// epilogue's per-chunk hand-over went from ~385 to ~1250 cycles with it).  For hand-overs whose
-// payload is NOT in memory written by this thread — tensor-memory stores already waited for, or
-// bulk copies whose completion this thread observed on an mbarrier.
-__device__ __forceinline__ void mbar_arrive_cluster_relaxed(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait_cluster(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-// converged wait on a barrier that threads of the peer CTA arrive on
-__device__ __forceinline__ void mbar_wait_converged_cluster(uint32_t bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!__all_sync(0xffffffffu, mbar_try_wait_cluster(bar, parity))) {
-    if (++spins > (1u << 24)) {
-      if ((threadIdx.x & 31) == 0)
-        printf("fsnerf: pair mbarrier timeout blk %d thr %d bar %u parity %u\n", blockIdx.x, threadIdx.x, bar, parity);
-      __trap();
-    }
-  }
-}
 __device__ __forceinline__ void bulk_s2g(void* dst, uint32_t src_smem, uint32_t bytes) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst),
                "r"(src_smem), "r"(bytes)
@@ -218,19 +169,6 @@ __device__ __forceinline__ void tmem_relinquish() {
 }
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols)
-               : "memory");
-}
-// CTA-pair forms: the same warp of BOTH CTAs of the pair executes them
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t dst_smem, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem),
-               "r"(ncols)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish_pair() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols)
                : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() {
@@ -303,35 +241,6 @@ __device__ __forceinline__ bool elect_one() {
       "selp.u32 %0, 1, 0, p;\n\t}"
       : "=r"(pred));
   return pred != 0;
-}
-// cta_group::2: ONE instruction, issued by the leader CTA of a pair, computes M = 256 rows — 128
-// from each CTA's tensor memory (A, D at the same addresses in both) — against an N-wide B whose
-// two N/2 halves sit at the same shared-memory offset of the two CTAs: each SM fetches and holds
-// half of every weight operand.  Completions (commit) arrive on the barrier at the same offset in
-// BOTH CTAs.
-__device__ __forceinline__ void umma_bf16_ts_pair(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc,
-                                                  uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_bf16_ss_pair(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                                  uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-      "h"((uint16_t)3)
-      : "memory");
 }
 // Converged-issue forms: executed by ALL lanes of the issuing warp with a per-lane guard that is
 // true for one lane only.  In the micro-benchmark (tools/mma_bench.cu) the operands stayed in

@@ -34,7 +34,6 @@
 //  (images with two readers: += 1 each).  Neither poll sits on a critical path: the store
 //  warps fetch the next slot's counter while the current image is still being staged, and a
 //  scout warp of each wgrad CTA polls ahead of its bulk-copy issuers.
-#include <stdlib.h>
 #include "common.cuh"
 #include "mlp_common.cuh"
 #include "mlp_issue.cuh"
@@ -962,36 +961,22 @@ mlp_heads_wgrad_kernel(const __grid_constant__ HeadsArgs a) {
 // ------------------------------------------------------------------ host-side plan
 constexpr int kFlagBytes = 32768;  // prod [148] + cons [148][kMaxRingDepth] uint32, padded
 constexpr int kMaxRingDepth = 32;
-
-int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-// wgrad CTAs of the fused launch (FSNERF_BWD_WGRAD_CTAS) and ring slots per dgrad CTA
-// (FSNERF_BWD_RING_DEPTH): tuning knobs, read once
-int wgrad_ctas_wanted() {
-  static int v = -1;
-  if (v < 0) v = env_int("FSNERF_BWD_WGRAD_CTAS", 58);
-  return v;
-}
-int job_overhead_cycles() {
-  static int v = -1;
-  if (v < 0) v = env_int("FSNERF_BWD_JOB_OVERHEAD", 3000);
-  return v;
-}
+// CTAs of the fused launch that take the weight-gradient role: swept 54-62, all within 2 % (56 was
+// 1-2 % ahead of 58 on a fast box and behind on a slow one; profiles/README.md)
+constexpr int kWgradCtas = 58;
+// per-tile overhead of a wgrad job in the job cost model (see the cost comment in fsnerf_mlp_backward)
+constexpr int kJobOverheadCycles = 3000;
 // tile_of rows: a dgrad CTA may claim up to 4x its even share (then it stops claiming)
 int tile_row_cap(int64_t n_tiles, int n_d) { return (int)(4 * ((n_tiles + n_d - 1) / n_d) + 8); }
 int64_t tile_table_bytes(int64_t n_tiles, int n_d) {
   return (((int64_t)n_d * tile_row_cap(n_tiles, n_d) * 4) + 1023) & ~(int64_t)1023;
 }
 int ring_depth_for(int n_img) {
-  static int v = -1;
-  if (v < 0) v = env_int("FSNERF_BWD_RING_DEPTH", 0);
-  // default: half a tile's images.  The slots are rewritten every few microseconds and must stay
-  // in L2 against the stash and weight streams passing through it: measured 3.75 ms (5 slots,
-  // 29 MB for 90 dgrad CTAs) vs 4.06 ms (10 slots) vs 4.2 ms (20 slots) per C2 fused launch on the
-  // same box; below 4 the producers stall on their readers (2 slots: 4.04 ms)
-  int d = v > 0 ? v : (n_img + 1) / 2;
+  // half a tile's images.  The slots are rewritten every few microseconds and must stay in L2
+  // against the stash and weight streams passing through it: measured 3.75 ms (5 slots, 29 MB for
+  // 90 dgrad CTAs) vs 4.06 ms (10 slots) vs 4.2 ms (20 slots) per C2 fused launch on the same box;
+  // below 4 the producers stall on their readers (2 slots: 4.04 ms)
+  int d = (n_img + 1) / 2;
   if (d < 2) d = 2;
   if (d > kMaxRingDepth) d = kMaxRingDepth;
   return d;
@@ -1003,7 +988,7 @@ struct SplitB {
 // how the (at most) 148 CTAs of the fused launch divide into the two roles
 SplitB split_roles(int n_jobs, int64_t n_tiles) {
   SplitB s;
-  int n_w = wgrad_ctas_wanted();
+  int n_w = kWgradCtas;
   if (n_w < n_jobs) n_w = n_jobs;
   if (n_w > kNumSMs - 1) n_w = kNumSMs - 1;
   // a job never gets more CTAs than there are tiles
@@ -1165,7 +1150,7 @@ extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* param
       // cycles a wgrad CTA spends per tile: its MMAs (M = 128 per a-chunk pair, N = 64 per
       // b-chunk: N/2 cycles per K = 16 step, 8 steps per tile) plus a per-tile overhead that the
       // stage ring does not hide (swept 0-12000 cycles: 1500 is ~15 % slower, 3000 and up are flat)
-      cost[WP.n_jobs] = (J.a_chunks / 2) * 8 * (J.b_chunks * 32) + job_overhead_cycles();
+      cost[WP.n_jobs] = (J.a_chunks / 2) * 8 * (J.b_chunks * 32) + kJobOverheadCycles;
       total += cost[WP.n_jobs];
       ++WP.n_jobs;
     }

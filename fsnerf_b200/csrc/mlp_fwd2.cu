@@ -19,7 +19,6 @@
 //                thread do not overlap (tools/l2_bench.cu).
 // Training (kTrain): every A image (SW128 byte image, the format dgrad / wgrad load
 // back) is also staged through smem per 32-row slab and bulk-stored to the stash.
-#include <stdlib.h>
 #include "common.cuh"
 #include "mlp_common.cuh"
 #include "mlp_encode.cuh"
@@ -89,10 +88,9 @@ struct Fwd2Args {
   int density_only;
   float* out;
   uint8_t* stash;
-  int pair;  // launched as clusters of two CTAs whose MMAs are cta_group::2 (M = 256 over both SMs)
 };
 
-template <bool kTrain, bool kPair>
+template <bool kTrain>
 __global__ void __launch_bounds__(kThreads2, 1)
 mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__ Fwd2Args args,
                 const __grid_constant__ IssueTable tab) {
@@ -120,16 +118,7 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
   for (int g = 0; g < prog.n_hidden; ++g)
     if (prog.layer[g].use_aux) last_pos_user = g;
   const int64_t n_tiles = (args.n_samples + kTileM - 1) / kTileM;
-  // CTA pairs (args.pair): the two CTAs of a cluster work on two tiles as ONE M = 256 problem.
-  // Rank 0 issues tcgen05.mma.cta_group::2 for both; every weight operand is split by N between
-  // the two SMs' shared memories, so each SM fetches HALF the weight bytes per tile — the layer
-  // period of the single-CTA kernel is set by the 32 KB-per-chunk weight stream into the SM
-  // (~665 cycles per chunk at ~50 B/clk, measured), not by the 512 cycles of MMAs.  Both CTAs run
-  // the even CTA's iteration count; a tile index past the end is a dummy (computed, not stored).
-  constexpr bool pair = kPair;
-  const int pair_rank = pair ? (int)cluster_ctarank() : -1;
-  const TileSeq seq = TileSeq::strided((int64_t)blockIdx.x, (int64_t)gridDim.x, n_tiles,
-                                       (int64_t)blockIdx.x - (pair ? pair_rank : 0));
+  const TileSeq seq = TileSeq::strided((int64_t)blockIdx.x, (int64_t)gridDim.x, n_tiles);
 
   if ((sbase & 1023u) != 0) {
     if (threadIdx.x == 0) printf("fsnerf: dynamic smem base not 1024B aligned (%u)\n", sbase);
@@ -137,29 +126,23 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
   }
   if (threadIdx.x == 0) {
     for (int s = 0; s < kStages; ++s) {
-      mbar_init(bar_w_full + 8 * s, (pair && pair_rank == 0) ? 2 : 1);  // leader: + the peer's relay
+      mbar_init(bar_w_full + 8 * s, 1);
       mbar_init(bar_w_empty + 8 * s, 1);
     }
-    // the leader's operand barriers count the warps of both CTAs
-    for (int c = 0; c < 4; ++c) mbar_init(bar_a_ready + 8 * c, pair ? 2 * kEpiWarps : kEpiWarps);
+    for (int c = 0; c < 4; ++c) mbar_init(bar_a_ready + 8 * c, kEpiWarps);
     mbar_init(bar_acc_full, kMmaWarps);
     mbar_init(bar_acc_full + 8, kMmaWarps);
     mbar_init(bar_token, 1);
     mbar_init(bar_token + 8, 1);
-    mbar_init(bar_pos_full, pair ? 2 * kEncWarps : kEncWarps);
+    mbar_init(bar_pos_full, kEncWarps);
     mbar_init(bar_pos_empty, 1);
-    mbar_init(bar_dir_full, pair ? 2 * kEncWarps : kEncWarps);
+    mbar_init(bar_dir_full, kEncWarps);
     mbar_init(bar_dir_empty, 1);
     fence_barrier_init();
   }
   if (warp == kWarpMma) {
-    if constexpr (pair) {
-      tmem_alloc_pair(tmem_slot, kTmemCols2);
-      tmem_relinquish_pair();
-    } else {
-      tmem_alloc(tmem_slot, kTmemCols2);
-      tmem_relinquish();
-    }
+    tmem_alloc(tmem_slot, kTmemCols2);
+    tmem_relinquish();
   }
   // biases: constant bank -> shared memory (the epilogue reads them as broadcast LDS.128;
   // indexed constant loads miss the small constant cache and serialise the epilogue)
@@ -171,25 +154,21 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
     reinterpret_cast<float*>(smem + S::heads)[i] = __ldg(small + kSmallSigmaW + i);
   const float* head_b = reinterpret_cast<const float*>(smem + S::heads) + 640;
   tc_fence_before();
-  if (pair) cluster_sync_all();  // the peer's barriers are initialised before anything is sent to them
-  else __syncthreads();
+  __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot_ptr;
 
   if (warp >= kWarpProd0) {
     // ------------------------------------------------ weight producers
     IssueBars IB{bar_w_full, bar_w_empty, bar_token, sbase + S::ring};
-    producer_loop<kStages>(tab, IB, args.packed, seq, warp - kWarpProd0, lane, pair_rank);
+    producer_loop<kStages>(tab, IB, args.packed, seq, warp - kWarpProd0, lane);
   } else if (warp >= kWarpMma) {
     // ------------------------------------------------ MMA issuers (mlp_issue.cuh)
     // Within a layer the encoding chunk (smem operand, independent of the previous epilogue)
     // goes FIRST in the table: it fills the bubble while the epilogue converts chunk 0.
     if (tmem_base != 0) __trap();  // 512 columns = the whole tensor memory
     IssueBars IB{bar_w_full, bar_w_empty, bar_token, sbase + S::ring};
-    if (pair_rank <= 0)
-      issuer_loop<kStages, kPair>(tab, IB, sbase, seq, (uint32_t)(warp - kWarpMma), lane, args.trace);
-    else if (warp == kWarpMma)  // peer CTA: its MMAs are issued by the leader
-      weight_relay_loop<kStages>(tab, IB, seq, lane);
+    issuer_loop<kStages>(tab, IB, sbase, seq, (uint32_t)(warp - kWarpMma), lane, args.trace);
   } else if (warp >= kWarpEnc0) {
     // ------------------------------------------------ encoders (thread = sample row)
     const int row = (warp - kWarpEnc0) * 32 + lane;
@@ -197,7 +176,6 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
     for (int64_t tile; (tile = seq.get(titer)) >= 0; ++titer) {
       const int64_t p = tile * kTileM + row;
       const bool valid = p < args.n_samples;
-      const bool real = tile < n_tiles;
       float pos[3] = {0.f, 0.f, 0.f}, dir[3] = {0.f, 0.f, 0.f};
       if (valid) {
         if (args.x) {
@@ -229,9 +207,8 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
       fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) {
-        if (pair_rank > 0) mbar_arrive_cluster(cluster_map_shared(bar_pos_full, 0));  // release: the tile is in this CTA's smem
-        else mbar_arrive(bar_pos_full);
-        if (kTrain && real) {
+        mbar_arrive(bar_pos_full);
+        if (kTrain) {
           const int slab = (warp - kWarpEnc0) * kSlabBytes2;
           bulk_s2g(stash_tile + prog.stash_aux_pos_off + slab, sbase + S::aux_pos + slab, kSlabBytes2);
           bulk_commit();
@@ -244,9 +221,8 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) {
-          if (pair_rank > 0) mbar_arrive_cluster(cluster_map_shared(bar_dir_full, 0));
-          else mbar_arrive(bar_dir_full);
-          if (kTrain && real) {
+          mbar_arrive(bar_dir_full);
+          if (kTrain) {
             const int slab = (warp - kWarpEnc0) * kSlabBytes2;
             bulk_s2g(stash_tile + prog.stash_aux_dir_off + slab, sbase + S::aux_dir + slab, kSlabBytes2);
             bulk_commit();
@@ -263,14 +239,12 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
     const uint32_t tmem_lane = tmem_base + ((uint32_t)(quarter * 32) << 16);
     const uint32_t stage_base = sbase + S::staging + quarter * (kStageBufs * kSlabBytes2);
     const bool issuer = kTrain && half == 0 && lane == 0;
-    const uint32_t a_ready_leader = pair ? cluster_map_shared(bar_a_ready, 0) : bar_a_ready;
     uint32_t acc_phase = 0;  // bit r: parity of accumulator region r (a register, not a local array)
     uint32_t n_staged = 0;
     uint32_t titer = 0;
     for (int64_t tile; (tile = seq.get(titer)) >= 0; ++titer) {
       const int64_t p = tile * kTileM + row;
       const bool valid = p < args.n_samples;
-      const bool real = tile < n_tiles;
       uint8_t* stash_tile = kTrain ? args.stash + (size_t)tile * prog.stash_tile_bytes : nullptr;
       float sigma = 0.f;
       for (int g = 0; g < n_gemm; ++g) {
@@ -280,6 +254,8 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
         const bool last = (g == n_gemm - 1);
         const int epi = L.epi;
         const int nchunk = L.n_halves * 2;
+        // this layer's ReLU mask words in the tile's stash record (null: the layer has none)
+        uint8_t* const mask_tile = (kTrain && L.mask_off >= 0) ? stash_tile + L.mask_off : nullptr;
         if (threadIdx.x == 0) FS_TRACE2(titer, g, 3);
         mbar_wait(bar_acc_full + 8 * r, (acc_phase >> r) & 1u);
         acc_phase ^= 1u << r;
@@ -343,20 +319,16 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
             tmem_st_wait();
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) {
-              // (the operand is in tensor memory and its store has been waited for: no memory release)
-              if (pair_rank > 0) mbar_arrive_cluster_relaxed(a_ready_leader + 8 * c);
-              else mbar_arrive(bar_a_ready + 8 * c);
-            }
+            if (lane == 0) mbar_arrive(bar_a_ready + 8 * c);
           }
           if (kTrain) {
-            if (L.mask_off >= 0 && real) {
+            if (mask_tile) {
               // 1-bit ReLU mask of these 32 features (what dgrad reads instead of the activations):
               // one word per row, 128 B per warp store
               uint32_t bits = 0;
 #pragma unroll
               for (int q = 0; q < 16; ++q) bits = relu_bits_fold(bits, w[q], q);
-              *reinterpret_cast<uint32_t*>(stash_tile + L.mask_off + relu_bits_word_off(c, half, row)) = bits;
+              *reinterpret_cast<uint32_t*>(mask_tile + relu_bits_word_off(c, half, row)) = bits;
             }
             // SW128 image slab of this quarter's 32 rows of chunk c -> stash
             const uint32_t buf = stage_base + (n_staged % kStageBufs) * kSlabBytes2;
@@ -367,7 +339,7 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
             fence_proxy_async_smem();
             if (issuer) bulk_wait_read1();  // slabs older than the previous one have been read
             named_bar_sync(1 + quarter, 64);
-            if (issuer && real) {
+            if (issuer) {
               bulk_s2g(stash_tile + L.stash_off + c * kChunkBytes + quarter * kSlabBytes2, buf, kSlabBytes2);
               bulk_commit();
             }
@@ -400,12 +372,8 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
     if (issuer) bulk_wait0();
   }
   tc_fence_before();
-  if (pair) cluster_sync_all();  // the peer's last commits arrive on this CTA's barriers: stay until it is done
-  else __syncthreads();
-  if (warp == kWarpMma) {
-    if constexpr (pair) tmem_dealloc_pair(tmem_base, kTmemCols2);
-    else tmem_dealloc(tmem_base, kTmemCols2);
-  }
+  __syncthreads();
+  if (warp == kWarpMma) tmem_dealloc(tmem_base, kTmemCols2);
 }
 
 }  // namespace
@@ -419,15 +387,11 @@ int mlp_forward_v2(const MlpProgram& P, const void* packed, int64_t n_samples, i
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 64 || !configured[dev]) {
-      cudaError_t e1 = cudaFuncSetAttribute(mlp_fwd2_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+      cudaError_t e1 = cudaFuncSetAttribute(mlp_fwd2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                             Smem<false>::total);
-      cudaError_t e2 = cudaFuncSetAttribute(mlp_fwd2_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+      cudaError_t e2 = cudaFuncSetAttribute(mlp_fwd2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                             Smem<true>::total);
-      cudaError_t e3 = cudaFuncSetAttribute(mlp_fwd2_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            Smem<false>::total);
-      cudaError_t e4 = cudaFuncSetAttribute(mlp_fwd2_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            Smem<true>::total);
-      for (cudaError_t e : {e1, e2, e3, e4})
+      for (cudaError_t e : {e1, e2})
         if (e != cudaSuccess) {
           fsnerf_set_error("mlp_forward: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
           return FSNERF_ERR_CUDA;
@@ -444,9 +408,6 @@ int mlp_forward_v2(const MlpProgram& P, const void* packed, int64_t n_samples, i
   a.density_only = density_only; a.out = out; a.stash = reinterpret_cast<uint8_t*>(stash);
   FS_REQUIRE(P.n_gemm <= kMaxLayers2, "mlp_forward: at most %d GEMM layers are supported", kMaxLayers2);
   const int64_t n_tiles = (n_samples + kTileM - 1) / kTileM;
-  static const int pair_env = [] { const char* e = getenv("FSNERF_FWD_PAIR"); return e ? atoi(e) : 0; }();
-  const bool pair_launch = pair_env != 0 && n_tiles >= 2;
-  a.pair = pair_launch ? 1 : 0;
   IssueTable T;
   T.pad = 0;
   {
@@ -483,7 +444,7 @@ int mlp_forward_v2(const MlpProgram& P, const void* packed, int64_t n_samples, i
           if (is_dir) R.xbar = bar(Bars<true>::dir_empty, Bars<false>::dir_empty);
           else if (g == last_pos_user) R.xbar = bar(Bars<true>::pos_empty, Bars<false>::pos_empty);
         }
-        R.idesc = umma_idesc_bf16(pair_launch ? 256 : 128, L.n_halves == 2 ? 256 : 128, 0, 0);
+        R.idesc = umma_idesc_bf16(128, L.n_halves == 2 ? 256 : 128, 0, 0);
         R.accbar = bar(Bars<true>::acc_full, Bars<false>::acc_full) + 8 * (g & 1);
         R.n_acc = issue_n_acc(i, nch);
         R.w_block = (uint32_t)(L.first_block + (c >= 0 ? c : L.n_act_chunks) * L.n_halves);
@@ -498,34 +459,12 @@ int mlp_forward_v2(const MlpProgram& P, const void* packed, int64_t n_samples, i
     for (int g = 0; g < n_gemm; ++g)
       if ((g & 1) == ((n_gemm - 1) & 1)) ++T.last_acc_n;
   }
-  int grid = (int)(n_tiles < kNumSMs ? n_tiles : kNumSMs);
-  if (a.pair) grid = (grid + 1) & ~1;  // whole pairs (kNumSMs is even); the odd CTA may run dummies only
+  const int grid = (int)(n_tiles < kNumSMs ? n_tiles : kNumSMs);
   FsProfScope prof_(stash ? "mlp_fwd_train" : "mlp_fwd", stream);
-  {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(kThreads2);
-    cfg.dynamicSmemBytes = stash ? Smem<true>::total : Smem<false>::total;
-    cfg.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = a.pair ? 2 : 1;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    cudaError_t e;
-    if (a.pair)
-      e = stash ? cudaLaunchKernelEx(&cfg, mlp_fwd2_kernel<true, true>, P, a, T)
-                : cudaLaunchKernelEx(&cfg, mlp_fwd2_kernel<false, true>, P, a, T);
-    else
-      e = stash ? cudaLaunchKernelEx(&cfg, mlp_fwd2_kernel<true, false>, P, a, T)
-                : cudaLaunchKernelEx(&cfg, mlp_fwd2_kernel<false, false>, P, a, T);
-    if (e != cudaSuccess) {
-      fsnerf_set_error("mlp_forward: launch: %s", cudaGetErrorString(e));
-      return FSNERF_ERR_CUDA;
-    }
-  }
+  if (stash)
+    mlp_fwd2_kernel<true><<<grid, kThreads2, Smem<true>::total, (cudaStream_t)stream>>>(P, a, T);
+  else
+    mlp_fwd2_kernel<false><<<grid, kThreads2, Smem<false>::total, (cudaStream_t)stream>>>(P, a, T);
   return fsnerf_check_launch("mlp_forward");
 }
 

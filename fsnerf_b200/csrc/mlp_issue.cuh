@@ -97,15 +97,12 @@ __host__ __device__ __forceinline__ uint32_t relu_bits_word_off(int chunk, int h
 // CTA claims tiles from a global counter a little ahead of their use and publishes them in shared
 // memory: feed[0] = tiles claimed so far (monotonic), feed[1 + (i & 3)] = tile of iteration i or -1
 // when the work has run out.  Every role warp asks for iteration i and gets the same answer.
-// A static sequence may run past n_tiles (CTA pairs sharing multicast weight stages must do the
-// same number of iterations): such a tile is a dummy — computed, never stored.
 struct TileSeq {
   volatile int* feed;
   int64_t first, stride, n_tiles;
   int64_t n_iters;  // static sequences only
-  __device__ __forceinline__ static TileSeq strided(int64_t first, int64_t stride, int64_t n_tiles, int64_t lead) {
-    // `lead`: the CTA whose iteration count this one follows (itself, or the even CTA of its pair)
-    const int64_t n = lead < n_tiles ? (n_tiles - lead + stride - 1) / stride : 0;
+  __device__ __forceinline__ static TileSeq strided(int64_t first, int64_t stride, int64_t n_tiles) {
+    const int64_t n = first < n_tiles ? (n_tiles - first + stride - 1) / stride : 0;
     return TileSeq{nullptr, first, stride, n_tiles, n};
   }
   __device__ __forceinline__ int64_t get(uint32_t titer) const {
@@ -134,15 +131,9 @@ struct TileSeq {
 
 // ------------------------------------------------------------------ weight producers
 // Producer `me` of kProdWarps streams every kProdWarps-th stage: L2 -> smem, one bulk copy.
-// pair_rank >= 0: this CTA is one of a cluster pair whose MMAs are cta_group::2 instructions issued
-// by rank 0.  Each CTA fetches ITS N-half of every weight operand (the packed image stores an
-// operand as N-halves of 128 rows, a 128-row operand as one block whose 64-row halves are its two
-// 8 KB halves) into its own ring; a stage is free in both CTAs when the leader's commit has
-// arrived (multicast).  The leader learns that the peer's half has landed from the peer's relay
-// warp (weight_relay_loop): its w_full barriers count two arrivals.
 template <int kStages>
 __device__ __forceinline__ void producer_loop(const IssueTable& tab, const IssueBars& B, const uint8_t* packed,
-                                              const TileSeq& seq, int me, int lane, int pair_rank = -1) {
+                                              const TileSeq& seq, int me, int lane) {
   uint32_t cnt = 0;
   for (uint32_t titer = 0; seq.get(titer) >= 0; ++titer) {
     for (int j = 0; j < tab.n; ++j, ++cnt) {
@@ -150,32 +141,11 @@ __device__ __forceinline__ void producer_loop(const IssueTable& tab, const Issue
       const uint32_t stage = cnt % kStages, phase = (cnt / kStages) & 1;
       mbar_wait_relaxed(B.w_empty + 8 * stage, phase ^ 1);
       if (lane == 0) {
-        uint32_t bytes = tab.rec[j].w_bytes;
-        const uint8_t* src = packed + (size_t)tab.rec[j].w_block * kBlockBytes;
-        if (pair_rank >= 0) {
-          bytes >>= 1;
-          src += (size_t)pair_rank * bytes;
-        }
+        const uint32_t bytes = tab.rec[j].w_bytes;
         mbar_arrive_expect_tx(B.w_full + 8 * stage, bytes);
-        bulk_g2s(B.ring + stage * kStageBytes, src, bytes, B.w_full + 8 * stage);
+        bulk_g2s(B.ring + stage * kStageBytes, packed + (size_t)tab.rec[j].w_block * kBlockBytes, bytes,
+                 B.w_full + 8 * stage);
       }
-      __syncwarp();
-    }
-  }
-}
-
-// Peer CTA of a pair (rank 1), one warp: as each of this CTA's weight halves lands, arrive on the
-// LEADER's barrier of that stage.
-template <int kStages>
-__device__ __forceinline__ void weight_relay_loop(const IssueTable& tab, const IssueBars& B, const TileSeq& seq,
-                                                  int lane) {
-  uint32_t cnt = 0;
-  const uint32_t leader_w_full = cluster_map_shared(B.w_full, 0);
-  for (uint32_t titer = 0; seq.get(titer) >= 0; ++titer) {
-    for (int j = 0; j < tab.n; ++j, ++cnt) {
-      const uint32_t stage = cnt % kStages, phase = (cnt / kStages) & 1;
-      mbar_wait(B.w_full + 8 * stage, phase);
-      if (lane == 0) mbar_arrive_cluster_relaxed(leader_w_full + 8 * stage);
       __syncwarp();
     }
   }
@@ -204,12 +174,9 @@ __device__ __forceinline__ void producer_loop_thread(const IssueTable& tab, cons
 // All 32 lanes of issuer `me` run this loop in lock step on provably uniform values; the
 // tcgen05 instructions are guarded so that lane 0 alone issues them.  trace: optional
 // clock64 timeline [tile iteration < 4][layer][k]: k = 0 layer reached, 1 first MMA, 2 committed.
-// kPair: the cta_group::2 forms (a kernel that contains them can only be launched as clusters of
-// two, so the single-CTA kernels must not instantiate this path).
-template <int kStages, bool kPair = false>
+template <int kStages>
 __device__ __forceinline__ void issuer_loop(const IssueTable& tab, const IssueBars& B, uint32_t sbase,
                                             const TileSeq& seq, uint32_t me, int lane, long long* trace) {
-  constexpr bool pair = kPair;
   const int n_rec = tab.n;
   uint32_t titer = 0;
   int j = (int)me;
@@ -227,13 +194,8 @@ __device__ __forceinline__ void issuer_loop(const IssueTable& tab, const IssueBa
     const uint32_t b0 = umma_desc_lo(B.ring + stage * kStageBytes);
     const uint32_t apar = (((flags & kRecParTile) ? titer : 0u) ^ (flags >> kRecParShift)) & 1u;
     if (tr && first && titer < 4) trace[(titer * 16 + g_cur) * 8 + 0] = clock64();
-    if constexpr (pair) {  // (the peer CTA's relay, epilogue and encoder warps arrive on these too)
-      mbar_wait_converged_cluster(B.w_full + 8 * stage, wpar);
-      mbar_wait_converged_cluster(sbase + R.abar, apar);
-    } else {
-      mbar_wait_converged(B.w_full + 8 * stage, wpar);
-      mbar_wait_converged(sbase + R.abar, apar);
-    }
+    mbar_wait_converged(B.w_full + 8 * stage, wpar);
+    mbar_wait_converged(sbase + R.abar, apar);
     mbar_wait_converged(B.token + 8 * me, tok_par);  // the other issuer has queued its chunk
     tok_par ^= 1u;
     tc_fence_after();
@@ -241,19 +203,7 @@ __device__ __forceinline__ void issuer_loop(const IssueTable& tab, const IssueBa
     const uint32_t n_acc = R.n_acc;
     const uint32_t acc0 = first ? 0u : 1u;
     if (elect_one()) {  // one thread issues the chunk's MMAs, the hand-over and the completion arrivals
-      if constexpr (pair) {
-        if (is_tmem) {
-          umma_bf16_ts_pair(d_col, a0, umma_desc_from_lo(b0), idesc, acc0);
-          umma_bf16_ts_pair(d_col, a0 + 8, umma_desc_from_lo(b0 + 2), idesc, 1u);
-          umma_bf16_ts_pair(d_col, a0 + 32, umma_desc_from_lo(b0 + 4), idesc, 1u);
-          umma_bf16_ts_pair(d_col, a0 + 40, umma_desc_from_lo(b0 + 6), idesc, 1u);
-        } else {
-          umma_bf16_ss_pair(d_col, umma_desc_from_lo(a0), umma_desc_from_lo(b0), idesc, acc0);
-          umma_bf16_ss_pair(d_col, umma_desc_from_lo(a0 + 2), umma_desc_from_lo(b0 + 2), idesc, 1u);
-          umma_bf16_ss_pair(d_col, umma_desc_from_lo(a0 + 4), umma_desc_from_lo(b0 + 4), idesc, 1u);
-          umma_bf16_ss_pair(d_col, umma_desc_from_lo(a0 + 6), umma_desc_from_lo(b0 + 6), idesc, 1u);
-        }
-      } else if (is_tmem) {  // features [0,32) of the chunk at columns +0, +8; [32,64) at +32, +40
+      if (is_tmem) {  // features [0,32) of the chunk at columns +0, +8; [32,64) at +32, +40
         umma_bf16_ts(d_col, a0, umma_desc_from_lo(b0), idesc, acc0);
         umma_bf16_ts(d_col, a0 + 8, umma_desc_from_lo(b0 + 2), idesc, 1u);
         umma_bf16_ts(d_col, a0 + 32, umma_desc_from_lo(b0 + 4), idesc, 1u);
@@ -265,20 +215,11 @@ __device__ __forceinline__ void issuer_loop(const IssueTable& tab, const IssueBa
         umma_bf16_ss(d_col, umma_desc_from_lo(a0 + 6), umma_desc_from_lo(b0 + 6), idesc, 1u);
       }
       mbar_arrive(B.token + 8 * (me ^ 1u));  // the last MMA is queued: hand over
-      if constexpr (pair) {  // completions arrive in both CTAs
-        umma_commit_pair(B.w_empty + 8 * stage);
-        if (R.xbar) umma_commit_pair(sbase + R.xbar);
-        if (n_acc) {
-          umma_commit_pair(sbase + R.accbar);
-          if (n_acc > 1) umma_commit_pair(sbase + R.accbar);
-        }
-      } else {
-        umma_commit(B.w_empty + 8 * stage);
-        if (R.xbar) umma_commit(sbase + R.xbar);
-        if (n_acc) {
-          umma_commit(sbase + R.accbar);
-          if (n_acc > 1) umma_commit(sbase + R.accbar);
-        }
+      umma_commit(B.w_empty + 8 * stage);
+      if (R.xbar) umma_commit(sbase + R.xbar);
+      if (n_acc) {
+        umma_commit(sbase + R.accbar);
+        if (n_acc > 1) umma_commit(sbase + R.accbar);
       }
     }
     __syncwarp();

@@ -11,7 +11,6 @@
 after a deliberate change of the stash format or of the forward's arithmetic)."""
 import hashlib
 import os
-import subprocess
 import sys
 
 import numpy as np
@@ -137,19 +136,6 @@ def test_nothing_written_past_the_last_tile(dev, P):
     nb = ops.mlp_stash_bytes(cfg, P)
     assert bool((buf[nb:] == 0x3C).all())
     assert bool((buf[:nb] != 0x3C).any())
-
-
-@pytest.mark.gpu
-def test_stash_under_cta_pairs():
-    """The same checks with the forward launched as CTA pairs (FSNERF_FWD_PAIR=1, read once per
-    process, so in a child process)."""
-    if not torch.cuda.is_available():
-        pytest.skip("no CUDA device")
-    env = dict(os.environ, FSNERF_FWD_PAIR="1")
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-x", "-q", "-m", "gpu",
-                        "-k", "not cta_pairs"], cwd=ROOT, env=env, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, (r.stdout[-3000:], r.stderr[-1000:])
-    assert " passed" in r.stdout
 
 
 if __name__ == "__main__":

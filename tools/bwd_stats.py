@@ -33,7 +33,7 @@ g_ = trace.cpu()[6144:6144 + 2 * 148].view(148, 2).double()
 g_ = g_[g_[:, 0] > 0]
 print(f"last launch on the global timer: first CTA start -> last CTA end {(g_[:, 1].max() - g_[:, 0].min()) / 1e6:.3f} ms; "
       f"start spread {(g_[:, 0].max() - g_[:, 0].min()) / 1e3:.1f} us; end spread {(g_[:, 1].max() - g_[:, 1].min()) / 1e3:.1f} us")
-n_w = int(os.environ.get("FSNERF_BWD_WGRAD_CTAS", "58"))  # must match the library default when unset
+n_w = 58  # kWgradCtas in csrc/mlp_bwd2.cu
 n_d = 148 - n_w
 dg, wg = s[:n_d], s[n_d:]
 print(f"dgrad CTAs ({n_d}), kcycles mean [min..max]:")
