@@ -58,6 +58,8 @@ SIGNATURES = {
     "fsnerf_mlp_forward": (_i, [C.POINTER(NetCfg), _p, _p, _l, _i, _p, _p, _p, _p, _p, _p, _p, _p,
                                 _i, _p, _p, _p]),
     "fsnerf_mlp_backward": (_i, [C.POINTER(NetCfg), _p, _p, _l, _p, _p, _p, _i, _p, _p, _p]),
+    "fsnerf_mlp_bwd_workspace_bytes_deterministic": (_l, [C.POINTER(NetCfg), _l]),
+    "fsnerf_mlp_backward_deterministic": (_i, [C.POINTER(NetCfg), _p, _p, _l, _p, _p, _p, _i, _p, _p, _p]),
     "fsnerf_mse_loss_grad": (_i, [_l, _p, _p, _f, _p, _p, _p]),
     "fsnerf_profile_enable": (_i, [_i]),
     "fsnerf_profile_read": (_i, [_i, C.c_char_p, C.POINTER(_f), C.POINTER(_i)]),
@@ -65,6 +67,8 @@ SIGNATURES = {
     "fsnerf_adam_step": (_i, [_l, _p, _p, _p, _p, _f, _f, _f, _f, _i, _p]),
     "fsnerf_adam_step_reg": (_i, [_l, _p, _p, _p, _p, _f, _f, _f, _f, _i, _i, _f, _i,
                                  C.POINTER(_l), C.POINTER(_l), _p, _p]),
+    "fsnerf_adam_step_reg_deterministic": (_i, [_l, _p, _p, _p, _p, _f, _f, _f, _f, _i, _i, _f, _i,
+                                               C.POINTER(_l), C.POINTER(_l), _p, _p]),
 }
 
 _lib = None

@@ -73,10 +73,12 @@ class _NeRFFunction(torch.autograd.Function):
         if d_out is None:
             return (None,) * (4 + len(module._layout))
         grads = torch.zeros_like(module._flat)
-        ws = torch.empty(ops.mlp_bwd_workspace_bytes(module.cfg, ctx.P), dtype=torch.uint8,
+        # torch.use_deterministic_algorithms(True) selects the bitwise reproducible backward
+        det = torch.are_deterministic_algorithms_enabled()
+        ws = torch.empty(ops.mlp_bwd_workspace_bytes(module.cfg, ctx.P, det), dtype=torch.uint8,
                          device=out.device)
         ops.mlp_backward(module.cfg, module._flat, ctx.packed, ctx.P, ctx.stash, out,
-                         d_out.contiguous(), grads, ws)
+                         d_out.contiguous(), grads, ws, deterministic=det)
         module._last_flat_grad = grads
         views = [grads[o:o + n].view(p.shape) for (o, n), p in zip(module._layout, module._param_list())]
         return (None, None, None, None, *views)

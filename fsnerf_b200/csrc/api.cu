@@ -229,11 +229,13 @@ extern "C" int fsnerf_adam_step(int64_t n, float* params, const float* grads, fl
   return fsnerf_check_launch("adam_step");
 }
 
-extern "C" int fsnerf_adam_step_reg(int64_t n, float* params, const float* grads, float* m, float* v,
-                                    float lr, float beta1, float beta2, float eps, int step,
-                                    int reg_mode, float reg_alpha, int n_segs,
-                                    const int64_t* seg_begin, const int64_t* seg_end,
-                                    float* seg_sums, void* stream) {
+// norm_blocks: blocks per regularised tensor in the norm pass.  16 spread each sum over the GPU;
+// 1 gives each sum one fixed order (its block adds once to the zeroed sum), so the update is
+// reproducible bit for bit.
+static int adam_step_reg_impl(int64_t n, float* params, const float* grads, float* m, float* v, float lr,
+                              float beta1, float beta2, float eps, int step, int reg_mode, float reg_alpha,
+                              int n_segs, const int64_t* seg_begin, const int64_t* seg_end, float* seg_sums,
+                              int norm_blocks, void* stream) {
   FS_REQUIRE(params && grads && m && v, "adam_step_reg: null pointer");
   FS_REQUIRE(step >= 1, "adam_step_reg: step counts from 1");
   FS_REQUIRE(reg_mode == 1 || reg_mode == 2, "adam_step_reg: reg_mode must be 1 (l1) or 2 (l2)");
@@ -256,8 +258,26 @@ extern "C" int fsnerf_adam_step_reg(int64_t n, float* params, const float* grads
   // seg_sums doubles as the value of the penalty: sum|w| (l1) or sum w^2 (l2) per tensor
   if (cudaMemsetAsync(seg_sums, 0, sizeof(float) * n_segs, st) != cudaSuccess)
     return fsnerf_check_launch("adam_step_reg(memset)");
-  reg_norm_kernel<<<dim3(16, n_segs), threads, 0, st>>>(segs, params, seg_sums);
+  reg_norm_kernel<<<dim3(norm_blocks, n_segs), threads, 0, st>>>(segs, params, seg_sums);
   adam_reg_kernel<<<(unsigned)((n + threads - 1) / threads), threads, 0, st>>>(
       n, params, grads, m, v, step_size, beta1, beta2, eps, inv_sqrt_bc2, segs, seg_sums);
   return fsnerf_check_launch("adam_step_reg");
+}
+
+extern "C" int fsnerf_adam_step_reg(int64_t n, float* params, const float* grads, float* m, float* v,
+                                    float lr, float beta1, float beta2, float eps, int step,
+                                    int reg_mode, float reg_alpha, int n_segs,
+                                    const int64_t* seg_begin, const int64_t* seg_end,
+                                    float* seg_sums, void* stream) {
+  return adam_step_reg_impl(n, params, grads, m, v, lr, beta1, beta2, eps, step, reg_mode, reg_alpha, n_segs,
+                            seg_begin, seg_end, seg_sums, 16, stream);
+}
+
+extern "C" int fsnerf_adam_step_reg_deterministic(int64_t n, float* params, const float* grads, float* m,
+                                                  float* v, float lr, float beta1, float beta2, float eps,
+                                                  int step, int reg_mode, float reg_alpha, int n_segs,
+                                                  const int64_t* seg_begin, const int64_t* seg_end,
+                                                  float* seg_sums, void* stream) {
+  return adam_step_reg_impl(n, params, grads, m, v, lr, beta1, beta2, eps, step, reg_mode, reg_alpha, n_segs,
+                            seg_begin, seg_end, seg_sums, 1, stream);
 }

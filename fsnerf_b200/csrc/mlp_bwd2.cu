@@ -34,6 +34,13 @@
 //  (images with two readers: += 1 each).  Neither poll sits on a critical path: the store
 //  warps fetch the next slot's counter while the current image is still being staged, and a
 //  scout warp of each wgrad CTA polls ahead of its bulk-copy issuers.
+//
+//  Deterministic mode (kDet, fsnerf_mlp_backward_deterministic): the same kernels with every
+//  timing-dependent summation order fixed.  dgrad CTA b takes tiles b, b + n_d, ... (no tile
+//  counter); each wgrad CTA consumes its tiles in the fixed order (tile iteration, producer) and
+//  stores its dW with plain stores into its own workspace slot; the store warps keep private bias
+//  sums; the heads kernel writes per-block partials; one reduction kernel then adds every
+//  element's partials, in index order, to `grads`.  Every difference sits behind `if constexpr`.
 #include "common.cuh"
 #include "mlp_common.cuh"
 #include "mlp_issue.cuh"
@@ -139,6 +146,13 @@ struct WgradPlan {
   int n_jobs, n_ctas;
   WgradJob job[kMaxJobs];
 };
+// deterministic mode: the partial sums in the caller's workspace (unused by the default kernels)
+struct DetB {
+  float* wpart;                 // dW of every wgrad CTA: job j's CTA `part` at wpart_off[j] + part * nrows * ncols
+  int64_t wpart_off[kMaxJobs];  //   ([nrows x ncols] row-major, floats)
+  float* bpart;                 // bias sums [n_d][4 store warps][n_gemm][256]; warp 0's row ends as the CTA's total
+  int n_gemm;
+};
 
 constexpr int kSmemFused = SmemB::total > kWSmemTotal ? SmemB::total : kWSmemTotal;
 
@@ -197,9 +211,10 @@ struct StatClock {
 };
 
 // =========================================================================== dgrad role
+template <bool kDet>
 __device__ __forceinline__ void dgrad_cta(uint8_t* smem, const MlpProgram& prog, const PlanB& plan,
                                           const ArgsB& args, const IssueTable& tab, const RingB& ring,
-                                          const int my_id) {
+                                          const DetB& det, const int my_id) {
   const uint32_t sbase = smem_u32(smem);
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;  // (shuffle: provably warp-uniform)
   const uint32_t bar_w_full = sbase + BarsB::w_full;
@@ -218,9 +233,10 @@ __device__ __forceinline__ void dgrad_cta(uint8_t* smem, const MlpProgram& prog,
   // Tiles are claimed from a global counter (the ring manager keeps the feed two tiles ahead):
   // the dgrad CTAs do not run at the same speed (they are throttled by different wgrad CTAs and
   // sit at different distances from the L2 slices they stream from), a static split ends with
-  // the slowest one.
+  // the slowest one.  The deterministic mode takes that cost: CTA b takes tiles b, b + n_d, ...,
+  // so that the tiles behind each bias partial and each wgrad CTA's summation order are fixed.
   volatile int* feed = reinterpret_cast<volatile int*>(smem + BarsB::feed);
-  const TileSeq seq{feed, 0, 0, n_tiles};
+  const TileSeq seq = kDet ? TileSeq::strided(my_id, ring.n_d, n_tiles) : TileSeq{feed, 0, 0, n_tiles};
   long long* stats = args.trace ? args.trace + kStatBase + 8 * my_id : nullptr;
   const long long t_begin = stats ? clock64() : 0;
 
@@ -272,8 +288,12 @@ __device__ __forceinline__ void dgrad_cta(uint8_t* smem, const MlpProgram& prog,
         while (n_claimed < want) {
           int t = -1;
           if (!dry && n_claimed < ring.row_cap - 1) {
-            const int64_t c = atomicAdd(ring.tile_ctr, 1u);
-            if (c < n_tiles) t = (int)c;
+            if constexpr (kDet) {
+              t = (int)seq.get((uint32_t)n_claimed);  // static: the table still tells the scouts
+            } else {
+              const int64_t c = atomicAdd(ring.tile_ctr, 1u);
+              if (c < n_tiles) t = (int)c;
+            }
           }
           if (t < 0) dry = true;
           if (n_claimed < ring.row_cap) my_tiles[n_claimed] = t;  // read by the wgrad scouts after they acquire prod
@@ -336,6 +356,17 @@ __device__ __forceinline__ void dgrad_cta(uint8_t* smem, const MlpProgram& prog,
         for (int c = 0; c < nchunk; ++c, ++n_staged) {
           const uint32_t b = n_staged % kStageBufsB;
           const uint32_t buf = stage_base + b * kSlabBytesB;
+          // deterministic mode: this warp's own running bias sums (two columns per lane) live in
+          // the workspace: four private copies in shared memory would take 36 KB, 256 B more than
+          // the 227 KB a CTA can have.  Only this lane touches them, so plain loads and stores keep
+          // one fixed order; the load is issued before the slab wait to hide its latency.
+          float2* bsum = nullptr;
+          float2 bprev = make_float2(0.f, 0.f);
+          if constexpr (kDet) {
+            bsum = reinterpret_cast<float2*>(det.bpart + (((size_t)my_id * 4 + quarter) * det.n_gemm + layer) * 256 +
+                                             64 * c) + lane;
+            if (it > 0) bprev = *bsum;
+          }
           sc.start();
           mbar_wait_relaxed(bar_slab_full + 8 * (quarter * kStageBufsB + b), (n_staged / kStageBufsB) & 1);
           sc.stop(st_slab);
@@ -365,8 +396,12 @@ __device__ __forceinline__ void dgrad_cta(uint8_t* smem, const MlpProgram& prog,
             }
             // (a shared-memory float atomic is a CAS loop; four private copies with plain adds
             // measured the same 3.75 ms per launch and cost 36 KB: the store warps are not the limit)
-            atomicAdd(bias_acc + layer * 256 + 64 * c + 2 * lane, s0 + c0);
-            atomicAdd(bias_acc + layer * 256 + 64 * c + 2 * lane + 1, s1 + c1);
+            if constexpr (kDet) {
+              *bsum = make_float2(bprev.x + (s0 + c0), bprev.y + (s1 + c1));
+            } else {
+              atomicAdd(bias_acc + layer * 256 + 64 * c + 2 * lane, s0 + c0);
+              atomicAdd(bias_acc + layer * 256 + 64 * c + 2 * lane + 1, s1 + c1);
+            }
           }
           __syncwarp();
           if (lane == 0) mbar_arrive(bar_slab_free + 8 * (quarter * kStageBufsB + b));
@@ -524,16 +559,32 @@ __device__ __forceinline__ void dgrad_cta(uint8_t* smem, const MlpProgram& prog,
   __syncthreads();
   if (stats && threadIdx.x == 0) stats[0] = clock64() - t_begin;
   if (warp == kWarpMmaB) tmem_dealloc(tmem_base, 512);
-  for (int g = 0; g < prog.n_gemm; ++g) {  // bias gradients of this CTA -> global
-    const int ncols = prog.layer[g].n_halves * 128;
-    if ((int)threadIdx.x < ncols)
-      atomicAdd(args.grads + prog.layer[g].bias_off + threadIdx.x, bias_acc[g * 256 + threadIdx.x]);
+  if constexpr (kDet) {
+    // the four store warps' sums, combined in warp order into warp 0's row: this CTA's partial
+    // (the barrier above made their global stores visible to the whole CTA)
+    const size_t wstride = (size_t)det.n_gemm * 256;
+    float* mine = det.bpart + (size_t)my_id * 4 * wstride;
+    for (int g = 0; g < prog.n_gemm; ++g) {
+      const int ncols = prog.layer[g].n_halves * 128;
+      if ((int)threadIdx.x < ncols) {
+        float* p = mine + g * 256 + threadIdx.x;
+        p[0] = ((p[0] + p[wstride]) + p[2 * wstride]) + p[3 * wstride];
+      }
+    }
+  } else {
+    for (int g = 0; g < prog.n_gemm; ++g) {  // bias gradients of this CTA -> global
+      const int ncols = prog.layer[g].n_halves * 128;
+      if ((int)threadIdx.x < ncols)
+        atomicAdd(args.grads + prog.layer[g].bias_off + threadIdx.x, bias_acc[g * 256 + threadIdx.x]);
+    }
   }
 }
 
 // =========================================================================== wgrad role
+template <bool kDet>
 __device__ __forceinline__ void wgrad_cta(uint8_t* smem, const MlpProgram& prog, const ArgsB& args,
-                                          const WgradPlan& plan, const RingB& ring, const int cta) {
+                                          const WgradPlan& plan, const RingB& ring, const DetB& det,
+                                          const int cta) {
   const uint32_t sbase = smem_u32(smem);
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;  // (shuffle: provably warp-uniform)
   const uint32_t bar_full = sbase + kWSmemBars;
@@ -673,6 +724,82 @@ __device__ __forceinline__ void wgrad_cta(uint8_t* smem, const MlpProgram& prog,
           }
         }
       }
+    } else if (warp == 0 && kDet) {
+      // deterministic scout: the queue takes this CTA's tiles in the fixed order (tile iteration,
+      // producer index), waiting for the next one in that order even when others are ready, so the
+      // MMA warp adds them into tensor memory in a fixed sequence.  Lane l watches the l-th entry
+      // not yet queued; the ready prefix is appended.
+      //   No deadlock: every consumer follows the same global order and every producer writes its
+      // images in order.  Take the smallest (iteration, producer) pair not fully consumed.  Each of
+      // its readers has consumed everything smaller, so it waits for this pair and nothing else.
+      // The producer's first image of the pair needs a slot freed by an image of an earlier
+      // iteration (all consumed); image k of the pair needs the slot of image k - depth, an
+      // earlier image of the same pair or of an earlier iteration, which its readers can land as
+      // soon as it is published.  So the pair completes, and by induction every pair does.
+      //   Watchdogs: the longest wait here is one producer's next image (at most one launch's
+      // length, milliseconds); the bounds below, like the dgrad side's slot wait, are ~0.3 s or more
+      // of no progress.
+      const int64_t n_tiles = (args.n_samples + kTileM - 1) / kTileM;
+      uint32_t enq = 0, idle = 0;
+      for (uint32_t it = 0;; ++it) {
+        // producers of this CTA with a tile in iteration it: b = part + k n_split with
+        // b + it n_d < n_tiles (static tiles), a prefix k < K of the list since b grows with k
+        const int64_t left = n_tiles - (int64_t)it * ring.n_d - part;
+        int K = left <= 0 ? 0 : (int)((left + J.n_split - 1) / J.n_split);
+        if (K > n_mine) K = n_mine;
+        if (K <= 0) break;
+        const uint32_t need = it * (uint32_t)ring.n_img + (uint32_t)J.a_img + 1u;
+        for (int k0 = 0; k0 < K; k0 += 32) {
+          const int cnt = (K - k0 < 32) ? K - k0 : 32;
+          const int b = part + (k0 + lane) * J.n_split;
+          bool ready = lane >= cnt;
+          int32_t t = -1;
+          for (int done = 0; done < cnt;) {
+            if (!ready && (int32_t)(ld_acquire_u32(ring.prod + b) - need) >= 0) {
+              t = ring.tile_of[(size_t)b * ring.row_cap + it];
+              if (t < 0) { printf("fsnerf: wgrad scout: no tile, blk %d producer %d iteration %u\n", blockIdx.x, b, it); __trap(); }
+              ready = true;
+            }
+            const uint32_t nready = ~__ballot_sync(0xffffffffu, ready);
+            const int upto = nready ? __ffs(nready) - 1 : 32;  // lanes below `upto` are all ready
+            const int n_new = (upto < cnt ? upto : cnt) - done;
+            if (n_new > 0) {
+              if (lane == 0) {  // room in the queue
+                uint32_t spins = 0;
+                while ((int32_t)(enq + (uint32_t)n_new - *released_upto) > kWQueue) {
+                  __nanosleep(64);
+                  if (++spins > (1u << 24)) { printf("fsnerf: wgrad queue timeout blk %d\n", blockIdx.x); __trap(); }
+                }
+              }
+              __syncwarp();
+              if (lane >= done && lane < done + n_new) {
+                const uint32_t pos = enq + (uint32_t)(lane - done);
+                queue[2 * (pos % kWQueue)] = (uint32_t)t;
+                queue[2 * (pos % kWQueue) + 1] = (uint32_t)b | (it << 8);
+              }
+              enq += (uint32_t)n_new;
+              done += n_new;
+              __syncwarp();
+              if (lane == 0) {
+                __threadfence_block();
+                *ready_upto = enq;
+              }
+              idle = 0;
+            } else {
+              __nanosleep(128);
+              if (++idle > (1u << 22)) {
+                if (lane == 0) printf("fsnerf: wgrad scout waited too long for producer %d, blk %d enq %u\n",
+                                      part + (k0 + done) * J.n_split, blockIdx.x, enq);
+                __trap();
+              }
+            }
+          }
+        }
+      }
+      if (lane == 0) {
+        __threadfence_block();
+        *final_count = enq;
+      }
     } else if (warp == 0) {
       // scout: every lane watches up to kScoutSlots of this CTA's producers and appends a tile to
       // the queue as soon as its image is published (at most one per producer per sweep)
@@ -775,10 +902,17 @@ __device__ __forceinline__ void wgrad_cta(uint8_t* smem, const MlpProgram& prog,
       __syncwarp();
       if (mc.on) { stats[3] = st_full; stats[4] = n_done; stats[6] = j; stats[5] = st_lat; }
     }
-    if (warp >= 2 && warp < 6 && *final_count != 0) {
+    if (warp >= 2 && warp < 6 && (kDet || *final_count != 0)) {
       const int quarter = warp & 3;
       mbar_wait(bar_acc_full, 0);
       tc_fence_after();
+      // deterministic mode: plain stores into this CTA's own slot (zeros if it was dealt no tile)
+      float* slot = nullptr;
+      bool none = false;
+      if constexpr (kDet) {
+        slot = det.wpart + det.wpart_off[j] + (int64_t)part * J.nrows * J.ncols;
+        none = *final_count == 0;
+      }
       // The accumulator tile of a warp is [32 rows (lanes) x 32 columns (registers)]; a straight
       // flush would issue atomics strided by a weight row (32 cache lines per instruction).  It is
       // transposed through shared memory instead: lane = column, one line per atomic.
@@ -794,10 +928,17 @@ __device__ __forceinline__ void wgrad_cta(uint8_t* smem, const MlpProgram& prog,
           for (int i = 0; i < 32; ++i) tr[lane * 33 + i] = __uint_as_float(v[i]);
           __syncwarp();
           if (c0 + lane < J.ncols) {
-            float* __restrict__ gcol = args.grads + J.w_off + J.col0 + c0 + lane;
+            if constexpr (kDet) {
+              float* __restrict__ pcol = slot + c0 + lane;
 #pragma unroll 8
-            for (int rr = 0; rr < 32; ++rr)
-              if (rbase + rr < J.nrows) atomicAdd(gcol + (size_t)(rbase + rr) * J.ld, tr[rr * 33 + lane]);
+              for (int rr = 0; rr < 32; ++rr)
+                if (rbase + rr < J.nrows) pcol[(size_t)(rbase + rr) * J.ncols] = none ? 0.f : tr[rr * 33 + lane];
+            } else {
+              float* __restrict__ gcol = args.grads + J.w_off + J.col0 + c0 + lane;
+#pragma unroll 8
+              for (int rr = 0; rr < 32; ++rr)
+                if (rbase + rr < J.nrows) atomicAdd(gcol + (size_t)(rbase + rr) * J.ld, tr[rr * 33 + lane]);
+            }
           }
         }
       }
@@ -809,10 +950,12 @@ __device__ __forceinline__ void wgrad_cta(uint8_t* smem, const MlpProgram& prog,
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
+template <bool kDet>
 __global__ void __launch_bounds__(kThreadsB, 1)
 mlp_bwd_fused_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__ PlanB plan,
                      const __grid_constant__ ArgsB args, const __grid_constant__ IssueTable tab,
-                     const __grid_constant__ WgradPlan wplan, const __grid_constant__ RingB ring) {
+                     const __grid_constant__ WgradPlan wplan, const __grid_constant__ RingB ring,
+                     const __grid_constant__ DetB det) {
   extern __shared__ __align__(1024) uint8_t smem[];
   if ((smem_u32(smem) & 1023u) != 0) __trap();
   // Roles by contiguous block ranges.  Consecutive block indices land on the two SMs of one TPC
@@ -833,9 +976,9 @@ mlp_bwd_fused_kernel(const __grid_constant__ MlpProgram prog, const __grid_const
     args.trace[6500 + lin] = (long long)smid;
   }
   if (is_d)
-    dgrad_cta(smem, prog, plan, args, tab, ring, id);
+    dgrad_cta<kDet>(smem, prog, plan, args, tab, ring, det, id);
   else
-    wgrad_cta(smem, prog, args, wplan, ring, id);
+    wgrad_cta<kDet>(smem, prog, args, wplan, ring, det, id);
   if (args.trace && threadIdx.x == 0) {
     unsigned long long t;
     asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
@@ -862,8 +1005,11 @@ __device__ __forceinline__ uint4 ldg_u4(const void* p) {
 // 256 threads: thread t owns 16-byte unit (t & 31) [= 8 features of chunk (t&31)>>3]
 // of the 256-wide h image and, if (t & 31) < 16, of the 128-wide hb image; the 8
 // row-groups (t >> 5) split the 128 rows.  Every load is a coalesced 16 B / lane.
+// kDet: no atomics; block b writes its sums to part[b * kHeadPart + ...] (kHeadPart layout below).
+constexpr int kHeadPart = 648;  // sigma_w [256], rgb_w [3][128], rgb_b [3], sigma_b, padding
+template <bool kDet>
 __global__ void __launch_bounds__(256, 3)
-mlp_heads_wgrad_kernel(const __grid_constant__ HeadsArgs a) {
+mlp_heads_wgrad_kernel(const __grid_constant__ HeadsArgs a, float* __restrict__ part) {
   __shared__ float4 dsm[kTileM];  // (dz0, dz1, dz2, dsigma) per row
   __shared__ float red[8][32][33];
   const int t = threadIdx.x, u = t & 31, rg = t >> 5;
@@ -935,26 +1081,69 @@ mlp_heads_wgrad_kernel(const __grid_constant__ HeadsArgs a) {
   for (int c = 0; c < 3; ++c)
 #pragma unroll
     for (int e = 0; e < 8; ++e) red[rg][u][8 + 8 * c + e] = acc_r[c][e];
+  if constexpr (kDet) {
+    if (u == 0) dsm[rg] = acc_b;  // (dsm is free: its last reader passed the barrier above)
+  }
   __syncthreads();
+  float* my = nullptr;
+  if constexpr (kDet) my = part + (size_t)blockIdx.x * kHeadPart;
   {
     // thread t -> feature t of h (sigma head): unit t>>3, element t&7
     float s = 0.f;
     for (int g = 0; g < 8; ++g) s += red[g][t >> 3][t & 7];
-    atomicAdd(a.g_sigma_w + t, s);
+    if constexpr (kDet) my[t] = s; else atomicAdd(a.g_sigma_w + t, s);
     if (t < 128) {
 #pragma unroll
       for (int c = 0; c < 3; ++c) {
         float r3 = 0.f;
         for (int g = 0; g < 8; ++g) r3 += red[g][t >> 3][8 + 8 * c + (t & 7)];
-        atomicAdd(a.g_rgb_w + c * 128 + t, r3);
+        if constexpr (kDet) my[256 + c * 128 + t] = r3; else atomicAdd(a.g_rgb_w + c * 128 + t, r3);
       }
     }
   }
-  if (u == 0) {
+  if constexpr (kDet) {
+    if (t == 0) {  // the row groups' bias sums in row-group order
+      float4 bs = dsm[0];
+      for (int g = 1; g < 8; ++g) {
+        const float4 d = dsm[g];
+        bs.x += d.x; bs.y += d.y; bs.z += d.z; bs.w += d.w;
+      }
+      my[640] = bs.x; my[641] = bs.y; my[642] = bs.z; my[643] = bs.w;
+    }
+  } else if (u == 0) {
     atomicAdd(a.g_rgb_b + 0, acc_b.x);
     atomicAdd(a.g_rgb_b + 1, acc_b.y);
     atomicAdd(a.g_rgb_b + 2, acc_b.z);
     atomicAdd(a.g_sigma_b, acc_b.w);
+  }
+}
+
+// =========================================================================== deterministic reduction
+// grads[i] = grads[i] + (sum of element i's partials in index order): the wgrad CTAs of its job,
+// the dgrad CTAs (biases) or the heads blocks.  One thread per element, so the order is fixed.
+struct RedSeg {
+  int64_t dst;          // float offset in grads of element (0, 0)
+  int64_t src;          // float offset in the partials of part 0's element (0, 0)
+  int64_t part_stride;  // floats between consecutive parts
+  int rows, cols, dst_ld, src_ld, n_parts;
+};
+constexpr int kMaxRedSegs = kMaxJobs + kMaxLayersB + 4;
+struct RedPlan {
+  int n;
+  RedSeg seg[kMaxRedSegs];
+};
+__global__ void __launch_bounds__(256)
+mlp_bwd_det_reduce_kernel(const __grid_constant__ RedPlan plan, const float* __restrict__ parts,
+                          float* __restrict__ grads) {
+  const RedSeg& S = plan.seg[blockIdx.y];
+  const int64_t n = (int64_t)S.rows * S.cols;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / S.cols, c = i % S.cols;
+    const float* p = parts + S.src + r * S.src_ld + c;
+    float s = p[0];
+    for (int k = 1; k < S.n_parts; ++k) s += p[(int64_t)k * S.part_stride];
+    float* g = grads + S.dst + r * S.dst_ld + c;
+    *g = *g + s;
   }
 }
 
@@ -1006,6 +1195,113 @@ int count_jobs(const MlpProgram& P) {
   return n;
 }
 
+int heads_grid(int64_t n_tiles) {
+  // one resident wave (3 CTAs per SM): 0.203 vs 0.218 ms per C2 step with two waves, 0.237 with three.
+  // (On the wgrad CTAs' idle warps the heads cost ~4800 CUDA-core cycles per tile, more than the
+  // jobs that stage their inputs can absorb: measured 6.4-9.4 ms per launch against 0.22 ms here.)
+  return (int)(n_tiles < 3 * kNumSMs ? n_tiles : 3 * kNumSMs);
+}
+
+// ---- wgrad plan: (layer, input part) jobs, CTAs split in proportion to their cycles per tile
+int build_wgrad_plan(const MlpProgram& P, int64_t n_tiles, WgradPlan& WP, SplitB& sp) {
+  WP.n_jobs = 0;
+  double cost[kMaxJobs], total = 0;
+  int readers[kMaxGemm];
+  for (int g = 0; g < P.n_gemm; ++g) readers[g] = (P.layer[g].n_act_chunks ? 1 : 0) + (P.layer[g].use_aux ? 1 : 0);
+  for (int g = 0; g < P.n_gemm; ++g) {
+    const GemmLayer& L = P.layer[g];
+    const int a_chunks = L.n_halves * 2;
+    for (int part = 0; part < 2; ++part) {
+      if (part == 0 && L.n_act_chunks == 0) continue;
+      if (part == 1 && !L.use_aux) continue;
+      FS_REQUIRE(WP.n_jobs < kMaxJobs, "mlp_backward: too many wgrad jobs");
+      WgradJob& J = WP.job[WP.n_jobs];
+      J.a_img = P.n_gemm - 1 - g; J.a_chunks = a_chunks;
+      J.w_off = L.w_off; J.ld = L.ld; J.nrows = L.n_halves * 128;
+      J.cons_inc = 2 / readers[g];
+      if (part == 0) {
+        J.b_off = P.layer[g - 1].stash_off; J.b_chunks = L.n_act_chunks;
+        J.col0 = 0; J.ncols = L.n_act_chunks * 64;
+      } else {
+        J.b_off = (L.epi == EPI_BRANCH) ? P.stash_aux_dir_off : P.stash_aux_pos_off;
+        J.b_chunks = 1; J.col0 = L.n_act_chunks * 64; J.ncols = L.ld - J.col0;
+      }
+      // cycles a wgrad CTA spends per tile: its MMAs (M = 128 per a-chunk pair, N = 64 per
+      // b-chunk: N/2 cycles per K = 16 step, 8 steps per tile) plus a per-tile overhead that the
+      // stage ring does not hide (swept 0-12000 cycles: 1500 is ~15 % slower, 3000 and up are flat)
+      cost[WP.n_jobs] = (J.a_chunks / 2) * 8 * (J.b_chunks * 32) + kJobOverheadCycles;
+      total += cost[WP.n_jobs];
+      ++WP.n_jobs;
+    }
+  }
+  sp = split_roles(WP.n_jobs, n_tiles);
+  // CTAs per job proportional to its per-tile cycles; every job must keep up with the dgrad CTAs
+  // (a late reader stalls them through the ring), so the CTAs left over by rounding go, one at a
+  // time, to the job with the most cycles per CTA
+  int n_cta[kMaxJobs], used = 0;
+  for (int jn = 0; jn < WP.n_jobs; ++jn) {
+    int n = (int)(sp.n_w * cost[jn] / total);
+    if (n < 1) n = 1;
+    if (n > sp.n_d) n = sp.n_d;  // a wgrad CTA serves whole dgrad CTAs
+    n_cta[jn] = n;
+    used += n;
+  }
+  while (used > sp.n_w) {  // rounding up the small jobs overshot: take from the best-served job
+    int best = -1;
+    for (int jn = 0; jn < WP.n_jobs; ++jn)
+      if (n_cta[jn] > 1 && (best < 0 || cost[jn] / n_cta[jn] < cost[best] / n_cta[best])) best = jn;
+    if (best < 0) break;
+    --n_cta[best];
+    --used;
+  }
+  while (used < sp.n_w) {
+    int best = -1;
+    for (int jn = 0; jn < WP.n_jobs; ++jn)
+      if (n_cta[jn] < sp.n_d && (best < 0 || cost[jn] / n_cta[jn] > cost[best] / n_cta[best])) best = jn;
+    if (best < 0) break;
+    ++n_cta[best];
+    ++used;
+  }
+  int begin = 0;
+  for (int jn = 0; jn < WP.n_jobs; ++jn) {
+    WP.job[jn].cta_begin = begin;
+    WP.job[jn].n_split = n_cta[jn];
+    begin += n_cta[jn];
+  }
+  WP.n_ctas = begin;
+  return FSNERF_OK;
+}
+
+// bytes of the default workspace: flags, tile table, dpre ring
+int64_t ring_workspace_bytes(const MlpProgram& P, const SplitB& sp, int64_t n_tiles) {
+  return (int64_t)kFlagBytes + tile_table_bytes(n_tiles, sp.n_d) +
+         (int64_t)sp.n_d * ring_depth_for(P.n_gemm) * kImgSlotBytes;
+}
+
+// Deterministic mode: the partial sums follow the default workspace (offsets in floats from
+// there, each region 1 KB aligned): dW of every wgrad CTA, the dgrad CTAs' bias sums
+// [n_d][4][n_gemm][256], the heads blocks' sums [hgrid][kHeadPart].
+struct DetLayout {
+  int64_t wpart_off[kMaxJobs];
+  int64_t bpart_off, hpart_off, n_floats;
+};
+DetLayout det_layout(const MlpProgram& P, const WgradPlan& WP, const SplitB& sp, int64_t n_tiles) {
+  DetLayout D;
+  auto align = [](int64_t f) { return (f + 255) & ~(int64_t)255; };
+  int64_t f = 0;
+  for (int jn = 0; jn < WP.n_jobs; ++jn) {
+    D.wpart_off[jn] = f;
+    f += (int64_t)WP.job[jn].n_split * WP.job[jn].nrows * WP.job[jn].ncols;
+  }
+  for (int jn = WP.n_jobs; jn < kMaxJobs; ++jn) D.wpart_off[jn] = f;
+  D.bpart_off = f = align(f);
+  f += (int64_t)sp.n_d * 4 * P.n_gemm * 256;
+  D.hpart_off = f = align(f);
+  f += (int64_t)heads_grid(n_tiles) * kHeadPart;
+  D.n_floats = align(f);
+  return D;
+}
+
 }  // namespace
 }  // namespace fs
 
@@ -1021,10 +1317,22 @@ extern "C" int64_t fsnerf_mlp_bwd_workspace_bytes(const fsnerf_net_cfg* cfg, int
          (int64_t)sp.n_d * ring_depth_for(P.n_gemm) * kImgSlotBytes;
 }
 
-extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* params,
-                                   const void* packed, int64_t n_samples, const void* stash,
-                                   const float* out, const float* d_out, int density_only,
-                                   float* grads, void* workspace, void* stream) {
+extern "C" int64_t fsnerf_mlp_bwd_workspace_bytes_deterministic(const fsnerf_net_cfg* cfg, int64_t n_samples) {
+  MlpProgram P;
+  if (build_program(cfg, &P) != FSNERF_OK) return -1;
+  if (n_samples <= 0) return kFlagBytes;
+  const int64_t n_tiles = (n_samples + kTileM - 1) / kTileM;
+  WgradPlan WP;
+  SplitB sp;
+  if (build_wgrad_plan(P, n_tiles, WP, sp) != FSNERF_OK) return -1;
+  return ring_workspace_bytes(P, sp, n_tiles) + 4 * det_layout(P, WP, sp, n_tiles).n_floats;
+}
+
+namespace {
+template <bool kDet>
+int mlp_backward_impl(const fsnerf_net_cfg* cfg, const float* params, const void* packed, int64_t n_samples,
+                      const void* stash, const float* out, const float* d_out, int density_only, float* grads,
+                      void* workspace, void* stream) {
   MlpProgram P;
   int rc = build_program(cfg, &P);
   if (rc != FSNERF_OK) return rc;
@@ -1049,7 +1357,8 @@ extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* param
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 64 || !configured[dev]) {
-      cudaError_t e = cudaFuncSetAttribute(mlp_bwd_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemFused);
+      cudaError_t e = cudaFuncSetAttribute(mlp_bwd_fused_kernel<kDet>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           kSmemFused);
       if (e != cudaSuccess) {
         fsnerf_set_error("mlp_backward: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
         return FSNERF_ERR_CUDA;
@@ -1059,6 +1368,25 @@ extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* param
   }
   const int64_t n_tiles = (n_samples + kTileM - 1) / kTileM;
 
+  // ---- wgrad plan and, in deterministic mode, where the partial sums go
+  WgradPlan WP;
+  SplitB sp;
+  rc = build_wgrad_plan(P, n_tiles, WP, sp);
+  if (rc != FSNERF_OK) return rc;
+  uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
+  float* parts = reinterpret_cast<float*>(ws + ring_workspace_bytes(P, sp, n_tiles));
+  DetLayout DL;
+  DetB det;
+  det.wpart = det.bpart = nullptr;
+  det.n_gemm = P.n_gemm;
+  for (int jn = 0; jn < kMaxJobs; ++jn) det.wpart_off[jn] = 0;
+  if constexpr (kDet) {
+    DL = det_layout(P, WP, sp, n_tiles);
+    det.wpart = parts;
+    for (int jn = 0; jn < kMaxJobs; ++jn) det.wpart_off[jn] = DL.wpart_off[jn];
+    det.bpart = parts + DL.bpart_off;
+  }
+
   // ---- heads (sigma / rgb head weight gradients)
   HeadsArgs ha;
   ha.stash = reinterpret_cast<const uint8_t*>(stash); ha.stash_tile_bytes = P.stash_tile_bytes;
@@ -1066,13 +1394,12 @@ extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* param
   ha.n_samples = n_samples; ha.n_tiles = n_tiles; ha.out = out; ha.d_out = d_out;
   ha.g_sigma_w = grads + P.sigma_w_off; ha.g_sigma_b = grads + P.sigma_b_off;
   ha.g_rgb_w = grads + P.rgb_w_off; ha.g_rgb_b = grads + P.rgb_b_off;
-  // one resident wave (3 CTAs per SM): 0.203 vs 0.218 ms per C2 step with two waves, 0.237 with three.
-  // (On the wgrad CTAs' idle warps the heads cost ~4800 CUDA-core cycles per tile, more than the
-  // jobs that stage their inputs can absorb: measured 6.4-9.4 ms per launch against 0.22 ms here.)
-  const int hgrid = (int)(n_tiles < 3 * kNumSMs ? n_tiles : 3 * kNumSMs);
+  const int hgrid = heads_grid(n_tiles);
   {
     FsProfScope prof_("mlp_heads_wgrad", stream);
-    mlp_heads_wgrad_kernel<<<hgrid, 256, 0, st>>>(ha);
+    float* hpart = nullptr;
+    if constexpr (kDet) hpart = parts + DL.hpart_off;
+    mlp_heads_wgrad_kernel<kDet><<<hgrid, 256, 0, st>>>(ha, hpart);
   }
   rc = fsnerf_check_launch("mlp_backward(heads)");
   if (rc != FSNERF_OK) return rc;
@@ -1123,80 +1450,11 @@ extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* param
   for (int s = 0; s < PL.n_steps; ++s)
     if ((s & 1) == ((PL.n_steps - 1) & 1)) ++T.last_acc_n;
 
-  // ---- wgrad plan: (layer, input part) jobs, CTAs split in proportion to their cycles per tile
-  WgradPlan WP;
-  WP.n_jobs = 0;
-  double cost[kMaxJobs], total = 0;
-  int readers[kMaxGemm];
-  for (int g = 0; g < P.n_gemm; ++g) readers[g] = (P.layer[g].n_act_chunks ? 1 : 0) + (P.layer[g].use_aux ? 1 : 0);
-  for (int g = 0; g < P.n_gemm; ++g) {
-    const GemmLayer& L = P.layer[g];
-    const int a_chunks = L.n_halves * 2;
-    for (int part = 0; part < 2; ++part) {
-      if (part == 0 && L.n_act_chunks == 0) continue;
-      if (part == 1 && !L.use_aux) continue;
-      FS_REQUIRE(WP.n_jobs < kMaxJobs, "mlp_backward: too many wgrad jobs");
-      WgradJob& J = WP.job[WP.n_jobs];
-      J.a_img = P.n_gemm - 1 - g; J.a_chunks = a_chunks;
-      J.w_off = L.w_off; J.ld = L.ld; J.nrows = L.n_halves * 128;
-      J.cons_inc = 2 / readers[g];
-      if (part == 0) {
-        J.b_off = P.layer[g - 1].stash_off; J.b_chunks = L.n_act_chunks;
-        J.col0 = 0; J.ncols = L.n_act_chunks * 64;
-      } else {
-        J.b_off = (L.epi == EPI_BRANCH) ? P.stash_aux_dir_off : P.stash_aux_pos_off;
-        J.b_chunks = 1; J.col0 = L.n_act_chunks * 64; J.ncols = L.ld - J.col0;
-      }
-      // cycles a wgrad CTA spends per tile: its MMAs (M = 128 per a-chunk pair, N = 64 per
-      // b-chunk: N/2 cycles per K = 16 step, 8 steps per tile) plus a per-tile overhead that the
-      // stage ring does not hide (swept 0-12000 cycles: 1500 is ~15 % slower, 3000 and up are flat)
-      cost[WP.n_jobs] = (J.a_chunks / 2) * 8 * (J.b_chunks * 32) + kJobOverheadCycles;
-      total += cost[WP.n_jobs];
-      ++WP.n_jobs;
-    }
-  }
-  const SplitB sp = split_roles(WP.n_jobs, n_tiles);
-  // CTAs per job proportional to its per-tile cycles; every job must keep up with the dgrad CTAs
-  // (a late reader stalls them through the ring), so the CTAs left over by rounding go, one at a
-  // time, to the job with the most cycles per CTA
-  int n_cta[kMaxJobs], used = 0;
-  for (int jn = 0; jn < WP.n_jobs; ++jn) {
-    int n = (int)(sp.n_w * cost[jn] / total);
-    if (n < 1) n = 1;
-    if (n > sp.n_d) n = sp.n_d;  // a wgrad CTA serves whole dgrad CTAs
-    n_cta[jn] = n;
-    used += n;
-  }
-  while (used > sp.n_w) {  // rounding up the small jobs overshot: take from the best-served job
-    int best = -1;
-    for (int jn = 0; jn < WP.n_jobs; ++jn)
-      if (n_cta[jn] > 1 && (best < 0 || cost[jn] / n_cta[jn] < cost[best] / n_cta[best])) best = jn;
-    if (best < 0) break;
-    --n_cta[best];
-    --used;
-  }
-  while (used < sp.n_w) {
-    int best = -1;
-    for (int jn = 0; jn < WP.n_jobs; ++jn)
-      if (n_cta[jn] < sp.n_d && (best < 0 || cost[jn] / n_cta[jn] > cost[best] / n_cta[best])) best = jn;
-    if (best < 0) break;
-    ++n_cta[best];
-    ++used;
-  }
-  int begin = 0;
-  for (int jn = 0; jn < WP.n_jobs; ++jn) {
-    WP.job[jn].cta_begin = begin;
-    WP.job[jn].n_split = n_cta[jn];
-    begin += n_cta[jn];
-  }
-  WP.n_ctas = begin;
-
   // ---- ring + flags in the caller's workspace
   RingB RG;
   RG.n_d = sp.n_d;
   RG.depth = ring_depth_for(P.n_gemm);
   RG.n_img = P.n_gemm;
-  uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
   RG.prod = reinterpret_cast<uint32_t*>(ws);
   RG.tile_ctr = RG.prod + 255;
   RG.cons = RG.prod + 256;
@@ -1222,13 +1480,63 @@ extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* param
   // per SM, at most 148 of them, launched cooperatively so that the driver refuses instead of
   // deadlocking if that ever does not hold
   const int grid = sp.n_d + WP.n_ctas;
-  void* kargs[] = {(void*)&P, (void*)&PL, (void*)&a, (void*)&T, (void*)&WP, (void*)&RG};
-  FsProfScope prof_("mlp_bwd_fused", stream);
-  cudaError_t e = cudaLaunchCooperativeKernel((const void*)mlp_bwd_fused_kernel, dim3(grid), dim3(kThreadsB), kargs,
-                                              (size_t)kSmemFused, st);
-  if (e != cudaSuccess) {
-    fsnerf_set_error("mlp_backward: cooperative launch of %d CTAs failed: %s", grid, cudaGetErrorString(e));
-    return FSNERF_ERR_CUDA;
+  void* kargs[] = {(void*)&P, (void*)&PL, (void*)&a, (void*)&T, (void*)&WP, (void*)&RG, (void*)&det};
+  {
+    FsProfScope prof_("mlp_bwd_fused", stream);
+    cudaError_t e = cudaLaunchCooperativeKernel((const void*)mlp_bwd_fused_kernel<kDet>, dim3(grid), dim3(kThreadsB),
+                                                kargs, (size_t)kSmemFused, st);
+    if (e != cudaSuccess) {
+      fsnerf_set_error("mlp_backward: cooperative launch of %d CTAs failed: %s", grid, cudaGetErrorString(e));
+      return FSNERF_ERR_CUDA;
+    }
   }
-  return fsnerf_check_launch("mlp_backward(fused)");
+  rc = fsnerf_check_launch("mlp_backward(fused)");
+  if (rc != FSNERF_OK || !kDet) return rc;
+
+  // ---- deterministic mode: every element's partials, in index order, added to grads once
+  RedPlan RP;
+  RP.n = 0;
+  int64_t most = 0;
+  auto seg = [&](int64_t dst, int64_t src, int64_t part_stride, int rows, int cols, int dst_ld, int src_ld,
+                 int n_parts) {
+    RedSeg& S = RP.seg[RP.n++];
+    S.dst = dst; S.src = src; S.part_stride = part_stride;
+    S.rows = rows; S.cols = cols; S.dst_ld = dst_ld; S.src_ld = src_ld; S.n_parts = n_parts;
+    if ((int64_t)rows * cols > most) most = (int64_t)rows * cols;
+  };
+  for (int jn = 0; jn < WP.n_jobs; ++jn) {  // weights: the job's wgrad CTAs in CTA order
+    const WgradJob& J = WP.job[jn];
+    seg(J.w_off + J.col0, DL.wpart_off[jn], (int64_t)J.nrows * J.ncols, J.nrows, J.ncols, J.ld, J.ncols, J.n_split);
+  }
+  for (int g = 0; g < P.n_gemm; ++g)  // biases: the dgrad CTAs in CTA order
+    seg(P.layer[g].bias_off, DL.bpart_off + g * 256, (int64_t)4 * P.n_gemm * 256, 1, P.layer[g].n_halves * 128, 0, 0,
+        sp.n_d);
+  // heads: the blocks in block order
+  seg(P.sigma_w_off, DL.hpart_off, kHeadPart, 1, 256, 0, 0, hgrid);
+  seg(P.rgb_w_off, DL.hpart_off + 256, kHeadPart, 1, 384, 0, 0, hgrid);
+  seg(P.rgb_b_off, DL.hpart_off + 640, kHeadPart, 1, 3, 0, 0, hgrid);
+  seg(P.sigma_b_off, DL.hpart_off + 643, kHeadPart, 1, 1, 0, 0, hgrid);
+  {
+    FsProfScope prof_("mlp_bwd_det_reduce", stream);
+    const int gx = (int)((most + 255) / 256 < 256 ? (most + 255) / 256 : 256);
+    mlp_bwd_det_reduce_kernel<<<dim3(gx, RP.n), 256, 0, st>>>(RP, parts, grads);
+  }
+  return fsnerf_check_launch("mlp_backward(deterministic reduction)");
+}
+}  // namespace
+
+extern "C" int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* params,
+                                   const void* packed, int64_t n_samples, const void* stash,
+                                   const float* out, const float* d_out, int density_only,
+                                   float* grads, void* workspace, void* stream) {
+  return mlp_backward_impl<false>(cfg, params, packed, n_samples, stash, out, d_out, density_only, grads, workspace,
+                                  stream);
+}
+
+extern "C" int fsnerf_mlp_backward_deterministic(const fsnerf_net_cfg* cfg, const float* params,
+                                                 const void* packed, int64_t n_samples, const void* stash,
+                                                 const float* out, const float* d_out, int density_only,
+                                                 float* grads, void* workspace, void* stream) {
+  return mlp_backward_impl<true>(cfg, params, packed, n_samples, stash, out, d_out, density_only, grads, workspace,
+                                 stream);
 }

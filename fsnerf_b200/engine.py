@@ -54,12 +54,17 @@ class HotPath:
     grid, fixed-step marching (render_step_size, near 0, far 1e10) with the transmittance visibility
     filter (early_stop_eps 1e-4, alpha_thre 0) on a density-only forward, then a training forward of
     the survivors.  Its train_step reads two sizes on the host: N (candidates) and M (survivors).
-    near / far / n_coarse / n_fine do not apply to it."""
+    near / far / n_coarse / n_fine do not apply to it.
+
+    deterministic=True: the MLP backward and the weight-norm penalty run in their deterministic
+    mode, so on one GPU two engines built from the same seed and fed the same rays hold bitwise
+    identical parameters, Adam moments, occupancy grid and renders after any number of steps
+    (same library build and GPU model).  The loss sums stay atomics: they are only reported."""
 
     def __init__(self, n_coarse=64, n_fine=128, near=2.0, far=6.0, white_bkgd=True, device="cuda",
                  n_layers=8, d_hidden=256, skip=(4,), n_freqs=10, n_freqs_dir=4, log_space=True,
                  seed=42, lr=5e-4, process_group=None, world_size=None, sampler="hierarchical",
-                 roi_aabb=None, grid_resolution=128, grid_levels=1, render_step_size=5e-3):
+                 roi_aabb=None, grid_resolution=128, grid_levels=1, render_step_size=5e-3, deterministic=False):
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise FsnerfError("HotPath: CUDA device required (no CPU path)")
@@ -67,6 +72,7 @@ class HotPath:
             raise FsnerfError(f"HotPath: unknown sampler {sampler!r} (hierarchical | occgrid)")
         ops.require_device(self.device.index if self.device.index is not None else torch.cuda.current_device())
         self.occgrid = sampler == "occgrid"
+        self.deterministic = bool(deterministic)
         self.n_coarse, self.n_fine = int(n_coarse), int(n_fine)
         self.near, self.far, self.white_bkgd = float(near), float(far), bool(white_bkgd)
         self.cfg = ops.make_cfg(n_layers, d_hidden, skip, n_freqs, n_freqs_dir, log_space)
@@ -314,10 +320,11 @@ class HotPath:
         d_raw_c, _ = ops.composite_backward(o["raw_c"].view(R, self.n_coarse, 4), o["ts_c"], o["te_c"], d_rgb_c,
                                             bkgd=self.bkgd, occ=None if self.hier else occ)
         # one ring for both passes (they run back to back on the stream): it stays L2 resident
-        ws_c = self._bytes("bwd_ws", max(ops.mlp_bwd_workspace_bytes(cfg, R * self.n_coarse),
-                                         ops.mlp_bwd_workspace_bytes(cfg, R * (self.n_coarse + self.n_fine))))
+        det = self.deterministic
+        ws_c = self._bytes("bwd_ws", max(ops.mlp_bwd_workspace_bytes(cfg, R * self.n_coarse, det),
+                                         ops.mlp_bwd_workspace_bytes(cfg, R * (self.n_coarse + self.n_fine), det)))
         ops.mlp_backward(cfg, self.net_params(0), self.packed[0], R * self.n_coarse, o["st_c"], o["raw_c"],
-                         d_raw_c.view(-1, 4), self.net_grads(0), ws_c)
+                         d_raw_c.view(-1, 4), self.net_grads(0), ws_c, deterministic=det)
         self.launches += 2 + 2  # mse, composite bwd, heads, fused dgrad+wgrad
         if self.hier:
             S = self.n_coarse + self.n_fine
@@ -326,7 +333,7 @@ class HotPath:
                                                 bkgd=self.bkgd, occ=occ)
             ws_f = ws_c
             ops.mlp_backward(cfg, self.net_params(1), self.packed[1], R * S, o["st_f"], o["raw_f"],
-                             d_raw_f.view(-1, 4), self.net_grads(1), ws_f)
+                             d_raw_f.view(-1, 4), self.net_grads(1), ws_f, deterministic=det)
             self.launches += 2 + 2  # mse, composite bwd, heads, fused dgrad+wgrad
         if self.world > 1:
             # the path's one real exchange: SUM of the flat fp32 gradient (both nets)
@@ -335,7 +342,8 @@ class HotPath:
             self.step += 1
             if weight_reg is not None:
                 ops.adam_step_reg(self.params, self.grads, self.m, self.v, self.lr if lr is None else lr,
-                                  self.step, weight_reg[0], weight_reg[1], self.reg_segs, self.reg_sums)
+                                  self.step, weight_reg[0], weight_reg[1], self.reg_segs, self.reg_sums,
+                                  deterministic=self.deterministic)
                 self.launches += 2
             else:
                 ops.adam_step(self.params, self.grads, self.m, self.v, self.lr if lr is None else lr, self.step)
@@ -373,9 +381,9 @@ class HotPath:
         if trained:
             d_raw, _ = ops.composite_packed_backward(o["raw"], o["ts"], o["te"], o["offsets"], o["trans"], d_rgb,
                                                      bkgd=self.bkgd)
-            ws = self._bytes("bwd_ws", ops.mlp_bwd_workspace_bytes(cfg, M))
+            ws = self._bytes("bwd_ws", ops.mlp_bwd_workspace_bytes(cfg, M, self.deterministic))
             ops.mlp_backward(cfg, self.net_params(0), self.packed[0], M, o["st"], o["raw"], d_raw, self.net_grads(0),
-                             ws)
+                             ws, deterministic=self.deterministic)
             self._reduced[-1:].fill_(float(M))
             self.launches += 3
         any_trained = trained
@@ -388,7 +396,8 @@ class HotPath:
                 self.step += 1
                 if weight_reg is not None:
                     ops.adam_step_reg(self.params, self.grads, self.m, self.v, self.lr if lr is None else lr,
-                                      self.step, weight_reg[0], weight_reg[1], self.reg_segs, self.reg_sums)
+                                      self.step, weight_reg[0], weight_reg[1], self.reg_segs, self.reg_sums,
+                                  deterministic=self.deterministic)
                     self.launches += 2
                 else:
                     ops.adam_step(self.params, self.grads, self.m, self.v, self.lr if lr is None else lr, self.step)

@@ -258,6 +258,10 @@ def packed_points(ray_indices, t_starts, t_ends, rays_o, rays_d, want_dirs=False
 
 def offsets_from_ray_indices(ray_indices, n_rays):
     """[R+1] int64 segment offsets of sorted packed ray indices"""
+    if torch.are_deterministic_algorithms_enabled():
+        # torch's CUDA bincount refuses to run in that mode; on sorted indices the offsets are
+        # also where each ray's run starts (first index >= r), the same integers
+        return torch.searchsorted(ray_indices, torch.arange(n_rays + 1, device=ray_indices.device))
     counts = torch.bincount(ray_indices, minlength=n_rays)
     offsets = torch.zeros(n_rays + 1, dtype=torch.int64, device=ray_indices.device)
     torch.cumsum(counts, 0, out=offsets[1:])
@@ -359,8 +363,11 @@ def mlp_stash_bytes(cfg, n_samples):
     return _lib.load().fsnerf_mlp_stash_bytes(C.byref(cfg), int(n_samples))
 
 
-def mlp_bwd_workspace_bytes(cfg, n_samples):
-    return _lib.load().fsnerf_mlp_bwd_workspace_bytes(C.byref(cfg), int(n_samples))
+def mlp_bwd_workspace_bytes(cfg, n_samples, deterministic=False):
+    """bytes of the workspace mlp_backward needs (deterministic: that mode's, which is larger)"""
+    lib = _lib.load()
+    fn = lib.fsnerf_mlp_bwd_workspace_bytes_deterministic if deterministic else lib.fsnerf_mlp_bwd_workspace_bytes
+    return fn(C.byref(cfg), int(n_samples))
 
 
 def mlp_pack(cfg, params, packed=None):
@@ -398,11 +405,16 @@ def mlp_forward(cfg, params, packed, *, rays_o=None, rays_d=None, t_starts=None,
 
 
 def mlp_backward(cfg, params, packed, n_samples, stash, out, d_out, grads, workspace,
-                 density_only=False):
-    check(_lib.load().fsnerf_mlp_backward(
+                 density_only=False, deterministic=False):
+    """Adds the MLP gradient to grads.  deterministic=True: bitwise reproducible gradients (same
+    inputs, library build and GPU model); the workspace must then have
+    mlp_bwd_workspace_bytes(cfg, n_samples, deterministic=True) bytes."""
+    lib = _lib.load()
+    name = "fsnerf_mlp_backward_deterministic" if deterministic else "fsnerf_mlp_backward"
+    check(getattr(lib, name)(
         C.byref(cfg), ptr(params), ptr(packed), int(n_samples), ptr(stash), ptr(out),
         ptr(_f32c(d_out, "d_out")), int(density_only), ptr(grads), ptr(workspace), _stream()),
-        "fsnerf_mlp_backward")
+        name)
     return grads
 
 
@@ -435,16 +447,18 @@ def reg_segments(cfg, n_nets=1):
 
 
 def adam_step_reg(params, grads, m, v, lr, step, mode, alpha, segments, seg_sums,
-                  beta1=0.9, beta2=0.999, eps=1e-8):
+                  beta1=0.9, beta2=0.999, eps=1e-8, deterministic=False):
     """Adam with the weight-norm penalty fused in; mode 'l1' or anything else (Frobenius),
-    like the reference's `args.reg` switch.  seg_sums [len(segments)] device floats."""
+    like the reference's `args.reg` switch.  seg_sums [len(segments)] device floats.
+    deterministic=True: the per-tensor sums are added in one fixed order (reproducible update)."""
     n = len(segments)
     b = (C.c_int64 * n)(*[s[0] for s in segments])
     e = (C.c_int64 * n)(*[s[1] for s in segments])
-    check(_lib.load().fsnerf_adam_step_reg(params.numel(), ptr(params), ptr(grads), ptr(m), ptr(v),
-                                           float(lr), beta1, beta2, eps, int(step),
-                                           1 if mode == "l1" else 2, float(alpha), n, b, e,
-                                           ptr(seg_sums), _stream()), "fsnerf_adam_step_reg")
+    name = "fsnerf_adam_step_reg_deterministic" if deterministic else "fsnerf_adam_step_reg"
+    check(getattr(_lib.load(), name)(params.numel(), ptr(params), ptr(grads), ptr(m), ptr(v),
+                                     float(lr), beta1, beta2, eps, int(step),
+                                     1 if mode == "l1" else 2, float(alpha), n, b, e,
+                                     ptr(seg_sums), _stream()), name)
 
 
 # -------------------------------------------------------------- profiling

@@ -81,8 +81,11 @@ class _RenderFunction(torch.autograd.Function):
             # extras["sigmas"] (src/run-nerf.py:260-264): added to the compositor's
             d_raw = d_raw.view(-1, 4).add_(d_raw_in.reshape(-1, 4))
         grads = torch.zeros_like(model._flat)
-        ws, wtok = _claim(model, "bwd_ws", ops.mlp_bwd_workspace_bytes(model.cfg, R * S), raw.device)
-        ops.mlp_backward(model.cfg, model._flat, ctx.packed, R * S, ctx.stash, raw, d_raw.view(-1, 4), grads, ws)
+        # torch.use_deterministic_algorithms(True) selects the bitwise reproducible backward
+        det = torch.are_deterministic_algorithms_enabled()
+        ws, wtok = _claim(model, "bwd_ws", ops.mlp_bwd_workspace_bytes(model.cfg, R * S, det), raw.device)
+        ops.mlp_backward(model.cfg, model._flat, ctx.packed, R * S, ctx.stash, raw, d_raw.view(-1, 4), grads, ws,
+                         deterministic=det)
         del wtok
         ctx.tok = ctx.stash = None  # the stash can be reused by the next forward
         model._last_flat_grad = grads  # parallel.allreduce_module_gradients reduces this buffer in one collective

@@ -236,6 +236,20 @@ int fsnerf_mlp_backward(const fsnerf_net_cfg* cfg, const float* params, const vo
                         const float* d_out, int density_only, float* grads, void* workspace,
                         void* stream);
 
+/* Deterministic mode of the backward.  For the same inputs, library build and GPU model, the
+ * gradients it adds to `grads` are bitwise identical from run to run (the default backward's
+ * summation order depends on timing: its last bits vary).  Same arguments and contract as
+ * fsnerf_mlp_backward (accumulated into, caller zeroes; density_only unsupported), with a larger
+ * workspace: fsnerf_mlp_bwd_workspace_bytes_deterministic(cfg, n_samples) bytes.  It adds each
+ * element once: grads[i] = grads[i] + total_i, where total_i sums the element's partials in a
+ * fixed order.  Three launches: heads, the fused kernel with fixed tile and accumulation orders,
+ * and that reduction.  Same values as the default up to fp32 rounding; slower (profiles/README.md). */
+int64_t fsnerf_mlp_bwd_workspace_bytes_deterministic(const fsnerf_net_cfg* cfg, int64_t n_samples);
+int fsnerf_mlp_backward_deterministic(const fsnerf_net_cfg* cfg, const float* params, const void* packed,
+                                      int64_t n_samples, const void* stash, const float* out,
+                                      const float* d_out, int density_only, float* grads,
+                                      void* workspace, void* stream);
+
 /* ---- train-step arithmetic (src/run-nerf.py:216-217,255-258,282-285) ---- */
 /* d_rgb = grad_scale*2*(rgb-gt); loss_sum += sum((rgb-gt)^2) (atomic; caller zeroes) */
 int fsnerf_mse_loss_grad(int64_t n, const float* rgb, const float* gt, float grad_scale,
@@ -257,6 +271,16 @@ int fsnerf_adam_step_reg(int64_t n, float* params, const float* grads, float* m,
                          float beta1, float beta2, float eps, int step, int reg_mode,
                          float reg_alpha, int n_segs, const int64_t* seg_begin,
                          const int64_t* seg_end, float* seg_sums, void* stream);
+/* fsnerf_adam_step_reg with a reproducible penalty: every per-tensor sum (seg_sums) is added in
+ * one fixed order, so seg_sums and, with reg_mode 2, the update are bitwise identical from run to
+ * run (same inputs, library build and GPU model).  With reg_mode 1 the update never reads the sums,
+ * so it is reproducible through either entry point.  Same arguments; the norm pass runs one block
+ * per tensor instead of sixteen. */
+int fsnerf_adam_step_reg_deterministic(int64_t n, float* params, const float* grads, float* m, float* v,
+                                       float lr, float beta1, float beta2, float eps, int step,
+                                       int reg_mode, float reg_alpha, int n_segs,
+                                       const int64_t* seg_begin, const int64_t* seg_end,
+                                       float* seg_sums, void* stream);
 
 /* ---- measurement aid (bench.py): per-kernel device time ------------------ */
 /* on != 0: start recording a cudaEvent pair around every kernel this library
