@@ -61,6 +61,7 @@ constexpr int kStagesB = 4;
 constexpr int kSlabBytesB = 32 * 128;
 constexpr int kStageBufsB = 3;
 constexpr int kMaxLayersB = 12;
+static_assert(kMaxHidden + 2 <= kMaxLayersB, "every network build_program accepts must fit the backward");
 constexpr int kImgSlotBytes = 4 * kChunkBytes;        // one ring slot: a [128 x 256] bf16 image
 
 struct SmemB {
@@ -1446,7 +1447,7 @@ int mlp_backward_impl(const fsnerf_net_cfg* cfg, const float* params, const void
   T.n = j;
   T.last_acc_off = BarsB::acc_full + 8 * ((PL.n_steps - 1) & 1);
   T.last_acc_n = 0;
-  T.pad = 0;
+  T.drained_off = 0;  // no dgrad chunk is kRecDrained
   for (int s = 0; s < PL.n_steps; ++s)
     if ((s & 1) == ((PL.n_steps - 1) & 1)) ++T.last_acc_n;
 

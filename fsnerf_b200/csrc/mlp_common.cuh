@@ -22,6 +22,9 @@ constexpr int kTileM = 128;          // samples per tile (UMMA M)
 constexpr int kBlockBytes = 16384;   // one [128 x 64] bf16 SW128 block
 constexpr int kChunkBytes = 16384;   // one K-chunk of an activation tile (128 rows x 128 B)
 constexpr int kMaxGemm = 16;
+// hidden layers build_program accepts; n_gemm = n_layers + 2 (connection, branch) must fit the
+// forward's and the backward's bias tables (static_asserts next to them)
+constexpr int kMaxHidden = 10;
 constexpr int kMaxFreqs = 10;        // 3*(1+2L) <= 64
 // "small params" block appended to the packed image: fp32 copies of every bias and
 // of the sigma / rgb head weights, contiguous so ONE device-to-device copy moves

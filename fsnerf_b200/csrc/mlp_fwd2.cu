@@ -37,6 +37,7 @@ constexpr int kSlabBytes2 = 32 * 128;              // 32 rows of one chunk image
 constexpr int kStageBufs = 3;                      // staging buffers per lane quarter
 constexpr int kTmemCols2 = 512;
 constexpr int kMaxLayers2 = 12;                    // GEMM layers whose biases fit the smem table
+static_assert(kMaxHidden + 2 <= kMaxLayers2, "every network build_program accepts must fit the forward");
 template <bool kTrain> __host__ __device__ constexpr int n_stages() { return kTrain ? 4 : 5; }
 template <bool kTrain> struct Smem {
   static constexpr int ring = 0;
@@ -63,6 +64,7 @@ template <bool kTrain> struct Bars {
   static constexpr int dir_empty = dir_full + 8;
   static constexpr int token = dir_empty + 8;       // [2] MMA issuers' hand-over
   static constexpr int tmem_slot = token + 16;
+  static constexpr int drained = tmem_slot + 8;     // the epilogue has read the tile's last accumulator
 };
 
 
@@ -138,6 +140,7 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
     mbar_init(bar_pos_empty, 1);
     mbar_init(bar_dir_full, kEncWarps);
     mbar_init(bar_dir_empty, 1);
+    mbar_init(sbase + B::drained, kEpiWarps);
     fence_barrier_init();
   }
   if (warp == kWarpMma) {
@@ -347,6 +350,11 @@ mlp_fwd2_kernel(const __grid_constant__ MlpProgram prog, const __grid_constant__
           }
         }
         if (threadIdx.x == 0) FS_TRACE2(titer, g, 5);
+        if (last && tab.drained_off) {  // every load of the last accumulator has completed (tmem_ld_wait)
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) mbar_arrive(sbase + tab.drained_off);
+        }
         if (epi == EPI_RELU_SIGMA) {
           if (half == 1) exch[row].w = sig_part;
           named_bar_sync(1 + quarter, 64);
@@ -409,7 +417,7 @@ int mlp_forward_v2(const MlpProgram& P, const void* packed, int64_t n_samples, i
   FS_REQUIRE(P.n_gemm <= kMaxLayers2, "mlp_forward: at most %d GEMM layers are supported", kMaxLayers2);
   const int64_t n_tiles = (n_samples + kTileM - 1) / kTileM;
   IssueTable T;
-  T.pad = 0;
+  T.drained_off = 0;
   {
     const bool train = stash != nullptr;
     const int n_gemm = density_only ? P.n_hidden : P.n_gemm;
@@ -454,6 +462,15 @@ int mlp_forward_v2(const MlpProgram& P, const void* packed, int64_t n_samples, i
       if (L.n_act_chunks) ++cons;
     }
     T.n = j;
+    // A tile's first layers (layer 0, then layer 1 if its encoding chunk comes first) are issued
+    // before any chunk waits for an epilogue of the tile.  The one of them that writes the
+    // accumulator region of the last layer (region (n_gemm - 1) & 1: layer 0 when n_gemm is odd)
+    // must wait until the epilogue has read the previous tile's last accumulator.
+    for (int k = 0; k < T.n && !(T.rec[k].flags & kRecTmem); ++k)
+      if ((int)((T.rec[k].flags >> 24) & 1u) == ((n_gemm - 1) & 1)) {
+        T.rec[k].flags |= kRecDrained;
+        T.drained_off = bar(Bars<true>::drained, Bars<false>::drained);
+      }
     T.last_acc_off = bar(Bars<true>::acc_full, Bars<false>::acc_full) + 8 * ((n_gemm - 1) & 1);
     T.last_acc_n = 0;
     for (int g = 0; g < n_gemm; ++g)

@@ -37,6 +37,9 @@ constexpr uint32_t kRecFirst = 1u << 17;     // first chunk of its layer: overwr
 constexpr uint32_t kRecParTile = 1u << 18;   // operand-barrier parity toggles with the tile iteration
 constexpr uint32_t kRecParShift = 19;        // bit 19: base parity of the operand barrier
 constexpr uint32_t kRecLast = 1u << 20;      // last chunk of its layer (trace only)
+// the chunk overwrites the accumulator region of the previous tile's last layer before any chunk
+// of its tile has waited for an epilogue: wait until the epilogue has read that accumulator
+constexpr uint32_t kRecDrained = 1u << 21;
 
 // One record per 64-wide K chunk of a tile, in consumption order.  The table is a kernel
 // parameter so the issuing warps read it with uniform loads.
@@ -56,7 +59,9 @@ struct IssueTable {
   int n;
   uint32_t last_acc_off;  // accumulator-full barrier of the tile's last layer (smem byte offset)
   uint32_t last_acc_n;    // layers per tile sharing that barrier
-  uint32_t pad;
+  // barrier the epilogue completes once per tile after reading the last layer's accumulator, which
+  // kRecDrained chunks wait for (smem byte offset; 0: no chunk needs it)
+  uint32_t drained_off;
   IssueRec rec[kMaxChunks2];
 };
 
@@ -196,6 +201,7 @@ __device__ __forceinline__ void issuer_loop(const IssueTable& tab, const IssueBa
     if (tr && first && titer < 4) trace[(titer * 16 + g_cur) * 8 + 0] = clock64();
     mbar_wait_converged(B.w_full + 8 * stage, wpar);
     mbar_wait_converged(sbase + R.abar, apar);
+    if ((flags & kRecDrained) && titer > 0) mbar_wait_converged(sbase + tab.drained_off, (titer - 1) & 1u);
     mbar_wait_converged(B.token + 8 * me, tok_par);  // the other issuer has queued its chunk
     tok_par ^= 1u;
     tc_fence_after();

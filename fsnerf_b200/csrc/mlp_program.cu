@@ -10,8 +10,8 @@ int build_program(const fsnerf_net_cfg* cfg, MlpProgram* P) {
   FS_REQUIRE(cfg && P, "net cfg: null");
   FS_REQUIRE(cfg->d_hidden == 256, "net cfg: d_hidden must be 256 (tcgen05 tile width), got %d",
              cfg->d_hidden);
-  FS_REQUIRE(cfg->n_layers >= 2 && cfg->n_layers + 2 <= kMaxGemm, "net cfg: n_layers must be in [2,%d]",
-             kMaxGemm - 2);
+  FS_REQUIRE(cfg->n_layers >= 2 && cfg->n_layers <= kMaxHidden, "net cfg: n_layers must be in [2,%d], got %d",
+             kMaxHidden, cfg->n_layers);
   FS_REQUIRE(cfg->n_freqs_pos >= 0 && cfg->n_freqs_pos <= kMaxFreqs, "net cfg: n_freqs_pos must be <= 10");
   FS_REQUIRE(cfg->n_freqs_dir >= 0 && cfg->n_freqs_dir <= kMaxFreqs, "net cfg: n_freqs_dir must be <= 10");
   FS_REQUIRE((cfg->skip_mask >> (cfg->n_layers - 1)) == 0,

@@ -360,14 +360,20 @@ def mlp_packed_bytes(cfg):
 
 
 def mlp_stash_bytes(cfg, n_samples):
-    return _lib.load().fsnerf_mlp_stash_bytes(C.byref(cfg), int(n_samples))
+    n = _lib.load().fsnerf_mlp_stash_bytes(C.byref(cfg), int(n_samples))
+    if n < 0:
+        check(-1, "fsnerf_mlp_stash_bytes")
+    return n
 
 
 def mlp_bwd_workspace_bytes(cfg, n_samples, deterministic=False):
     """bytes of the workspace mlp_backward needs (deterministic: that mode's, which is larger)"""
     lib = _lib.load()
-    fn = lib.fsnerf_mlp_bwd_workspace_bytes_deterministic if deterministic else lib.fsnerf_mlp_bwd_workspace_bytes
-    return fn(C.byref(cfg), int(n_samples))
+    name = "fsnerf_mlp_bwd_workspace_bytes_deterministic" if deterministic else "fsnerf_mlp_bwd_workspace_bytes"
+    n = getattr(lib, name)(C.byref(cfg), int(n_samples))
+    if n < 0:
+        check(-1, name)
+    return n
 
 
 def mlp_pack(cfg, params, packed=None):

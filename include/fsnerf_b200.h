@@ -177,7 +177,15 @@ int fsnerf_occgrid_binarize(int64_t n_cells, const float* occs, float threshold,
                             void* stream);
 
 /* ---- (2)+(3) NeRF MLP -------------------------------------------------- */
-/* Architecture of core.models.NeRF (src/core/models.py:57-109). */
+/* Architecture of core.models.NeRF (src/core/models.py:57-109).  Accepted ranges (every entry
+ * point refuses anything else with FSNERF_ERR_ARG):
+ *   n_layers     2 .. 10
+ *   d_hidden     256
+ *   skip_mask    bits 0 .. n_layers-2 only (no skip after the last hidden layer)
+ *   n_freqs_*    0 .. 10 (an encoding of at most 63 channels)
+ * The backward runs one weight-gradient job per (layer, input part) and takes at most 20 of
+ * them: n_layers + (number of skip bits) <= 17.  Deeper nets with more skips still run the
+ * forward (inference); fsnerf_mlp_backward refuses them. */
 typedef struct fsnerf_net_cfg {
   int n_layers;    /* hidden layers before the bottleneck (8)              */
   int d_hidden;    /* 256 (the tcgen05 path supports 256 only)             */

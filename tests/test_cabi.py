@@ -71,7 +71,7 @@ def test_flatten_state_dict_layout():
 
 
 def test_deep_network_is_rejected_before_the_pack_table_overflows():
-    """12 hidden layers need 205 operand blocks > the 192-entry pack table: an error, not a host overflow"""
+    """12 hidden layers (205 operand blocks > the 192-entry pack table): an error, not a host overflow"""
     from fsnerf_b200 import ops
     from fsnerf_b200._lib import FsnerfError
     cfg = ops.make_cfg(n_layers=12)

@@ -436,6 +436,24 @@ def test_standalone_positional_encoder(dev, golden):
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("log_space", [True, False])
+@pytest.mark.parametrize("L", [0, 1, 6])
+def test_standalone_positional_encoder_widths(dev, L, log_space):
+    """the encoder at the widths and spacings the non-default networks use, against the oracle"""
+    from fsnerf_b200.core.models import PositionalEncoder
+    from oracle import encoding as oenc
+    g = torch.Generator().manual_seed(L)
+    x = (torch.rand(1000, 3, generator=g) * 2 - 1) * 3
+    pe = PositionalEncoder(3, L, log_space)
+    assert pe.d_output == 3 * (1 + 2 * L)
+    ref = oenc.positional_encoding(x, L, log_space)
+    assert ref.shape == (1000, pe.d_output)
+    np.testing.assert_allclose(pe(x.to(dev)).cpu().numpy(), ref.numpy(), rtol=0, atol=1e-6)  # same fp32 arguments
+    m = torch.rand(pe.d_output, generator=g)
+    np.testing.assert_allclose(pe(x.to(dev), m.to(dev)).cpu().numpy(), (ref * m).numpy(), rtol=0, atol=1e-6)
+
+
+@pytest.mark.gpu
 def test_mlp_forward_sigma_slot_and_render_coarse_skip(dev):
     """density_only=2 writes exactly the sigma of the full forward into raw[:,3]; a hierarchical
     render whose coarse pass skips the view branch gives bit-identical fine samples and image."""
